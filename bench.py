@@ -1,6 +1,6 @@
 """Headline benchmark: volumes/sec at 512x512x320 (BASELINE.json: "MIM train step + embedding inference, 1/2/4/8 B200").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 ONE JSON line.  The headline (`value`, `e2e`, `roofline`) is the workload that has a collective and that the north star
 sets its scaling target on — BASELINE configs[2], the smb-vision-base MIM pre-training step (forward + norm-pix MSE loss +
@@ -15,6 +15,10 @@ are the `classification` and `vjepa_step` blocks.
 the classes the reference imports (src/run_mim.py:19-20, src/run_inference.py:12), UNMODIFIED and at full depth (12 + 4
 layers), fp32, sdpa backend, all host threads — on the same synthetic volume: real steps, no extrapolation; the number of
 steps actually run is what the line's `steps` says (bounded by a time budget, `steps_requested` keeps the driver's K).
+
+`--dump-outputs DIR` writes what each timed block returned in its last timed step as DIR/<name>.npy (fp32, rank 0; the
+large arrays as the same seeded sample of rows in every run, < 64 MB in all).  The inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -123,6 +127,39 @@ class ClockSampler:
             return dict(sm_mhz=None, sm_max_mhz=None, reasons=[], samples=0)
         busy = [v for v in sm if v > 0.5 * max(sm)] or sm
         return dict(sm_mhz=statistics.median(busy), sm_max_mhz=mx, reasons=sorted(reasons), samples=len(sm))
+
+
+# ------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------
+DUMP_LIMIT = 64 << 20
+
+
+def host(t):
+    """fp32 host copy of a device tensor."""
+    return t.detach().float().cpu().numpy()
+
+
+def sample_rows(t, rows):
+    """fp32 host copy of `rows` rows of t [..., C] (leading dims flattened), chosen by a fixed seed and kept in order, so
+    every run samples the same rows; all of them when there are no more than `rows`."""
+    import torch
+
+    t = t.detach().reshape(-1, t.shape[-1])
+    if t.shape[0] > rows:
+        idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values
+        t = t[idx.to(t.device)]
+    return host(t)
+
+
+def write_dump(out_dir, arrays):
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -254,7 +291,10 @@ def main():
     ap.add_argument("--no-cls", action="store_true")
     ap.add_argument("--no-vjepa", action="store_true")
     ap.add_argument("--no-cuda-graph", action="store_true", help="time the eager step (475 launches) instead of the CUDA-graph replay of forward + backward")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each timed block returned in its last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -343,7 +383,8 @@ def main():
     dp = DataParallelStep(model, optimizer=opt, cuda_graph=use_graph)
     # the same step launch by launch: the pass in which single kernels can be bracketed by CUDA events (roofline) and launches counted
     dp_eager = DataParallelStep(model, optimizer=opt) if use_graph else dp
-    steps = max(args.steps, 1)
+    steps = args.steps
+    dump = {} if args.dump_outputs and rank == 0 else None  # name -> host array, written by write_dump at the end
 
     # CUDA events around the dominant kernel (attention backward, 16 calls per step): the library records them on the launching
     # stream right before / after the main kernel (smbv_flash_attn_bwd_fused: the fused one-pass kernel + its combine pass;
@@ -385,11 +426,18 @@ def main():
     ops.flash_attn_bwd = bwd_spy
     ops.attn_bwd_event_source = ev_source
     losses = []
+    mim_out = []  # (loss, logits) of the latest MIM step
+
+    def mim_step(d):
+        mim_out.clear()  # the last step's outputs are freed before this step allocates its own
+        mim_out.extend(d.step(vol_dev, mp))
+        losses.append(mim_out[0].clone())
+
     # the event pass runs with the second-stream queue OFF (training.SideQueue, SMBV_WGRAD_STREAM=0): with it the weight-gradient GEMMs of
     # the previous layer share the SMs with the bracketed attention backward and its CUDA-event duration is no longer the kernel's own
     _side_prev = os.environ.get("SMBV_WGRAD_STREAM")
     os.environ["SMBV_WGRAD_STREAM"] = "0"
-    ms_single, _, launches, _ = timed(lambda: losses.append(dp_eager.step(vol_dev, mp)[0].clone()), steps, hook=bwd_hook, clocks=False)
+    ms_single, _, launches, _ = timed(lambda: mim_step(dp_eager), steps, hook=bwd_hook, clocks=False)
     if _side_prev is None:
         os.environ.pop("SMBV_WGRAD_STREAM")
     else:
@@ -398,11 +446,14 @@ def main():
     ops.flash_attn_bwd = _orig_bwd
     torch.cuda.synchronize()
     # the product's eager step (second stream on): launch by launch, no per-kernel events
-    ms_eager, wall_eager, _, clocks_eager = timed(lambda: losses.append(dp_eager.step(vol_dev, mp)[0].clone()), steps, clocks=True)
+    ms_eager, wall_eager, _, clocks_eager = timed(lambda: mim_step(dp_eager), steps, clocks=True)
     if use_graph:  # HEADLINE: the graph replay (the inputs are resident: vol_dev / mp are copied into the static buffers device to device)
-        ms_mim, wall_mim, _, clocks = timed(lambda: losses.append(dp.step(vol_dev, mp)[0].clone()), steps, clocks=True)
+        ms_mim, wall_mim, _, clocks = timed(lambda: mim_step(dp), steps, clocks=True)
     else:
         ms_mim, wall_mim, clocks = ms_eager, wall_eager, clocks_eager
+    if dump is not None:  # now: the steps of (1b) overwrite the graph's static loss / logits
+        dump["mim_loss"] = host(mim_out[0])
+        dump["mim_logits"] = sample_rows(mim_out[1], 1024)  # [13312 masked tokens, 4096] bf16 -> 1024 rows, 16 MB
     dk_ms = [a.elapsed_time(b) for a, b in ev_used]  # dK/dV kernel alone (library-recorded events); dQ runs beside it, so it is NOT an isolated time
     call_ms = [a.elapsed_time(b) for a, b in call_events]  # the whole call: prep + dK/dV || dQ + join
     call_fl = [8.0 * N * N * 64 * H for H, N in ev_shapes[:len(call_ms)]]
@@ -529,11 +580,17 @@ def main():
             else:
                 yield
 
+        inf_out = []
+
         def infer():
             with torch.no_grad():  # the reference's inference loop (src/run_inference.py:78-86); with grad enabled the forward would keep activations
-                return model.videomae(x_dev)
+                inf_out.clear()
+                inf_out.append(model.videomae(x_dev).last_hidden_state)
 
         ms_dev, wall_dev, il, _ = timed(infer, steps, hook=fwd_hook)
+        if dump is not None:
+            dump["inference_last_hidden_state"] = sample_rows(inf_out[0], 4096)  # [20480, 768] -> 4096 rows, 12 MB
+        inf_out.clear()
         attn_ms = [a.elapsed_time(b) for a, b in attn_events]
         attn_avg = sum(attn_ms) / max(len(attn_ms), 1)
         from smb_vision_b200.inference import EmbeddingRunner
@@ -580,19 +637,21 @@ def main():
     # =====================================================================================================================
     if not args.no_cls:
         try:
-            line["classification"] = bench_classification(timed, dev, world, rank, steps, pk, use_graph)
+            line["classification"] = bench_classification(timed, dev, world, rank, steps, pk, use_graph, dump)
         except Exception as e:  # a secondary block must not take the headline down
             line["classification"] = {"error": f"{type(e).__name__}: {e}"}
     # (4) BASELINE configs[4]: V-JEPA2-3D training step + the encoder forward at 512x512x320
     if not args.no_vjepa:
         try:
-            line.update(bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph))
+            line.update(bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph, dump))
         except Exception as e:
             line["vjepa_step"] = {"error": f"{type(e).__name__}: {e}"}
 
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         torch.cuda.empty_cache()
         line["cpu_baseline"] = cpu_baseline_mim()
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -608,7 +667,7 @@ def main():
         os._exit(0)
 
 
-def bench_classification(timed, dev, world, rank, steps, pk, use_graph=True):
+def bench_classification(timed, dev, world, rank, steps, pk, use_graph=True, dump=None):
     """src/run_classification.py:452-504 / scripts/training/run_cls.sh: smb-vision-base encoder, 224x224x160 = 1960 tokens, batch 4 per
     GPU, 2 additional features, 2 labels; forward + cross-entropy + backward + all-reduce + clip + AdamW."""
     import torch
@@ -630,13 +689,21 @@ def bench_classification(timed, dev, world, rank, steps, pk, use_graph=True):
     labels = torch.tensor([0, 1, 1, 0]).to(dev)
     opt = FusedAdamW(model, lr=5e-5, weight_decay=0.01, max_grad_norm=1.0)
     vol = model.videomae._volume(x)
-    losses = []
+    losses, last = [], []
+
+    def step(d):
+        last.clear()
+        last.extend(d.step(vol, feats, labels))
+        losses.append(last[0].clone())
+
     dp_eager = DataParallelStep(model, optimizer=opt)
-    ms_eager, _, launches, _ = timed(lambda: losses.append(dp_eager.step(vol, feats, labels)[0].clone()), steps)
+    ms_eager, _, launches, _ = timed(lambda: step(dp_eager), steps)
     ms = ms_eager
     if use_graph:  # 1975 launches of mostly 5-10 us kernels: the eager step is launch-bound, the graph replay is the product path
         dp = DataParallelStep(model, optimizer=opt, cuda_graph=True)
-        ms, _, _, _ = timed(lambda: losses.append(dp.step(vol, feats, labels)[0].clone()), steps)
+        ms, _, _, _ = timed(lambda: step(dp), steps)
+    if dump is not None:
+        dump["cls_loss"], dump["cls_logits"] = host(last[0]), host(last[1])
     N, d, L, mlp = 1960, 768, 12, 3072
     flops = 3 * B * (2 * N * 4096 * d + L * (2 * N * d * (3 * d + d + 2 * mlp) + 4 * N * N * 64 * 12))
     vps = world * B * steps / (ms / 1e3)
@@ -647,7 +714,7 @@ def bench_classification(timed, dev, world, rank, steps, pk, use_graph=True):
             "loss_first": float(losses[0]), "loss_last": float(losses[-1]), "losses": [round(float(v), 5) for v in losses[:12]]}
 
 
-def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True):
+def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True, dump=None):
     """src/run_vjepa.py:101-141 at the reference's own input size (384x384x256 = 9216 tokens, ViT-L 1024/16/24 + predictor 384/12/12,
     src/run_vjepa.py:73-84, facebook/vjepa2-vitl-fpc64-256), batch 1 per GPU: online forward (encoder on context tokens + predictor),
     momentum-target encoder forward, L1, backward, all-reduce, clip + AdamW, EMA update.  Plus the ViT-L encoder forward alone at 512x512x320."""
@@ -661,7 +728,6 @@ def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True):
     from smb_vision_b200.vjepa import B200VJEPA2Model
 
     out = {}
-    vsteps = max(min(steps, 5), 3)
     ai.register()
     T, S = 256, 384
     vc = VJEPA2Config(patch_size=16, crop_size=S, frames_per_clip=T, tubelet_size=16, in_chans=1)
@@ -678,14 +744,14 @@ def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True):
     x = batch["pixel_values_videos"].to(dev)
     ctx, tgt = [m.to(dev) for m in batch["context_mask"]], [m.to(dev) for m in batch["target_mask"]]
     losses = []
-    ms_eager, _, launches, _ = timed(lambda: losses.append(vjepa_step(model, target, opt, grads, x, ctx, tgt).clone()), vsteps, warmup=2)
+    ms_eager, _, launches, _ = timed(lambda: losses.append(vjepa_step(model, target, opt, grads, x, ctx, tgt).clone()), steps, warmup=2)
     ms, graph_note = ms_eager, "eager"
     if use_graph:
         try:  # forward + backward replayed from a CUDA graph (examples/train_vjepa.GraphedVJEPAStep); optimiser + EMA behind it
             from examples.train_vjepa import GraphedVJEPAStep
 
             gstep = GraphedVJEPAStep(model, target, opt, grads)
-            ms, _, _, _ = timed(lambda: losses.append(gstep(x, ctx, tgt).clone()), vsteps, warmup=2)
+            ms, _, _, _ = timed(lambda: losses.append(gstep(x, ctx, tgt).clone()), steps, warmup=2)
             graph_note = "CUDA graph of forward + backward, optimiser + EMA launched behind it"
             gstep._graphs.clear()
         except Exception as e:
@@ -694,7 +760,7 @@ def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True):
         "workload": "V-JEPA2-3D training step (BASELINE configs[4]): ViT-L encoder (1024/16/24) + predictor (384/12/12), 384x384x256 = 9216 tokens "
                     "(the reference's own input size), batch 1 per GPU: online forward on the context tokens + predictor, momentum-target forward, L1, backward, "
                     "gradient all-reduce, clip + AdamW, EMA update",
-        "value": world * vsteps / (ms / 1e3), "unit": UNIT, "ms_per_step": ms / vsteps, "eager_ms_per_step": ms_eager / vsteps, "launch_mode": graph_note,
+        "value": world * steps / (ms / 1e3), "unit": UNIT, "ms_per_step": ms / steps, "eager_ms_per_step": ms_eager / steps, "launch_mode": graph_note,
         "gpu_launches_ours": launches,
         "context_tokens": int(ctx[0].shape[1]), "target_tokens": int(tgt[0].shape[1]),
         "native": "everything: encoder forward + backward (online and momentum target), predictor forward + backward (context gather, position-sort index "
@@ -707,16 +773,22 @@ def bench_vjepa(timed, dev, world, rank, steps, pk, x_dev, use_graph=True):
     torch.manual_seed(1)
     with torch.device(dev):
         vmodel = B200VJEPA2Model(vc2, with_predictor=False).eval()
+    vj_out = []
+
     def vj_infer():
         with torch.no_grad():
-            return vmodel.get_vision_features(x_dev)
+            vj_out.clear()
+            vj_out.append(vmodel.get_vision_features(x_dev))
 
-    ms_vj, _, n_launch, _ = timed(vj_infer, vsteps, warmup=2)
+    ms_vj, _, n_launch, _ = timed(vj_infer, steps, warmup=2)
+    if dump is not None:
+        dump["vjepa_loss"] = host(losses[-1])
+        dump["vjepa_encoder_features"] = sample_rows(vj_out[0], 4096)  # [20480, 1024] -> 4096 rows, 16 MB
     VJ_FLOPS = 2 * 20480 * 4096 * 1024 + 24 * (2 * 20480 * 1024 * 12 * 1024 + 4 * 20480 * 20480 * 1024)
     out["vjepa_encoder"] = {"workload": "V-JEPA2-3D ViT-L (1024/16 heads/24 layers) encoder forward, 512x512x320 = 20480 tokens, batch 1/GPU, bf16, random init",
-                            "value": world * vsteps / (ms_vj / 1e3), "unit": UNIT, "ms_per_volume": ms_vj / vsteps, "gpu_launches": n_launch,
-                            "model_tflops_per_gpu": VJ_FLOPS * vsteps / (ms_vj / 1e3) / 1e12,
-                            "frac_of_sustained_peak": VJ_FLOPS * vsteps / (ms_vj / 1e3) / 1e12 / pk["tf_sust"]}
+                            "value": world * steps / (ms_vj / 1e3), "unit": UNIT, "ms_per_volume": ms_vj / steps, "gpu_launches": n_launch,
+                            "model_tflops_per_gpu": VJ_FLOPS * steps / (ms_vj / 1e3) / 1e12,
+                            "frac_of_sustained_peak": VJ_FLOPS * steps / (ms_vj / 1e3) / 1e12 / pk["tf_sust"]}
     return out
 
 
