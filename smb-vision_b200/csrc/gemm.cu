@@ -483,7 +483,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           float v[32];
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]) * alpha;
-          if (e.bias && slice == 0) {  // (K slices > 0 of a split tile add only their partial sums)
+          // (K slices > 0 of a split tile add only their partial sums.)  c0 < N: with N % 64 == 32 the second half of the last slab
+          // lies past N; its values are clipped by the TMA store, and bias[N .. N+31] may lie outside the caller's allocation
+          if (e.bias && slice == 0 && c0 < e.N) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
               const float4 bb = __ldg(reinterpret_cast<const float4*>(e.bias + c0) + i);
