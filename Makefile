@@ -8,12 +8,6 @@ OBJS      := $(patsubst $(CSRC)/%.cu,build/%.o,$(SRCS))
 NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC \
              -Xptxas -v --expt-relaxed-constexpr -Iinclude
 
-# `make clean && make DEV=1`: developer build with the kernel variants, knock-out and timeline-trace hooks of
-# profiles/r01_attn_notes.md (tools/run_attn.py variants, trace_attn_*.py); the release library has none of them.
-ifdef DEV
-NVCCFLAGS += -DSMBV_DEV_BUILD
-endif
-
 all: $(LIB)
 
 build/%.o: $(CSRC)/%.cu $(CSRC)/common.cuh include/smbv_b200.h

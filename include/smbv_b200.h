@@ -117,9 +117,9 @@ int smbv_gemm_ex(const smbv_gemm_ex_args* a, smbv_stream_t st);
  * (natural-log sum-exp of the scaled scores, saved for backward).  Online-softmax flash tiling on tcgen05/TMEM. */
 int smbv_flash_attn_fwd(const smbv_bf16* q, const smbv_bf16* k, const smbv_bf16* v, int B, int H, int N, float scale,
                         smbv_bf16* out, float* lse, smbv_stream_t st);
-/* same, with a kernel-variant selector (0 = default; 1/2 = first-generation kernel with V^T / V; 11-13 = exp2 emulation
- * shares) and an optional workspace of smbv_flash_attn_fwd_workspace_bytes(B,H,N) bytes: with it, the query-tile pairs of
- * a partial last wave are split over 2..8 CTAs by key range and merged by a combine kernel (wave-quantisation fix). */
+/* same, with an optional workspace of smbv_flash_attn_fwd_workspace_bytes(B,H,N) bytes: with it, the query-tile pairs of
+ * a partial last wave are split over 2..8 CTAs by key range and merged by a combine kernel (wave-quantisation fix).
+ * `variant` is reserved and must be 0; any other value is rejected with an argument error. */
 int64_t smbv_flash_attn_fwd_workspace_bytes(int B, int H, int N);
 int smbv_flash_attn_fwd_ex(const smbv_bf16* q, const smbv_bf16* k, const smbv_bf16* v, int B, int H, int N, float scale,
                            smbv_bf16* out, float* lse, int variant, void* workspace, int64_t workspace_bytes,

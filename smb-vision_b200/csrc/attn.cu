@@ -2,26 +2,23 @@
 // Semantics: eager_attention_forward, reference modeling_videomae.py:196-223 (softmax in fp32, probabilities cast
 // to the value dtype before P@V, output [B,N,H,64]).
 //
-// One CTA = 128 query rows of one (batch, head); it streams KV blocks of 128 keys:
-//   warp 0 lane 0 : TMA producer (Q once; K and V tiles through 3-stage mbarrier rings, 128B swizzle)
-//   warp 1 lane 0 : MMA issuer   S(j+1) = Q K(j+1)^T   (M128 N128 K64, SS)   -- issued one block ahead of
-//                                 O    += P(j) V(j)      (M128 N64  K128, SS)  -- the softmax (S double-buffered in TMEM)
-//   warps 4..7    : softmax, one query row per thread: tcgen05.ld S -> running max with lazy rescaling
-//                   (O is rescaled in TMEM only when the max grows by more than 2^8) -> P = exp2 -> bf16 -> smem
-//   TMEM columns  : S0 [0,128)  S1 [128,256)  O [256,320)
-#include <cstdlib>
-
+// flash_attn_fwd2_kernel: two query tiles (256 rows) per CTA, two softmax warpgroups, everything but K/V/Q in TMEM.
+//   warpgroup 0 : warp 0 lane 0 = TMA producer (Q once; K and V tiles through 4-stage mbarrier rings, 128B swizzle),
+//                 warp 1 / warp 2 lane 0 = MMA issuer of tile A / tile B
+//   warpgroup 1 : softmax of tile A (rows q0 .. q0+127), one row per thread;  warpgroup 2 : tile B
+//   TMEM        : S_A [0,128) S_B [128,256) | P_A [256,320) P_B [320,384) (bf16 pairs) | O_A [384,448) O_B [448,512)
+// The softmax releases S as soon as it sits in registers (s_free), so S(j+1) = Q K(j+1)^T is computed WHILE the
+// softmax of block j runs; P is written back to TMEM and feeds O += P V as the TMEM A operand (no smem round trip).
+// Each tile has its own issuing thread (blocking mbarrier waits in the tile's natural event order s_free, p_full, ...),
+// so neither tile queues behind the other's softmax.  Running max with lazy rescaling: O is rescaled in TMEM only when
+// the max grows by more than 2^8.  Packed f32x2 math (FFMA2/FADD2) + FMNMX3.
 #include "common.cuh"
 #include "../../include/smbv_b200.h"
 
 namespace smbv {
 
 constexpr int ATT_BQ = 128, ATT_BK = 128, ATT_D = 64;
-constexpr int ATT_KSTAGES = 3, ATT_VSTAGES = 3;
-constexpr int ATT_TILE_BYTES = 128 * 64 * 2;  // 16 KB: one [128 x 64] bf16 tile (Q, K, V or half of P)
-constexpr int ATT_P_BYTES = 2 * ATT_TILE_BYTES;
-constexpr int ATT_SMEM = ATT_TILE_BYTES * (1 + ATT_KSTAGES + ATT_VSTAGES) + 2 * ATT_P_BYTES + 1024 + 256;
-constexpr int ATT_THREADS = 256;
+constexpr int ATT_TILE_BYTES = 128 * 64 * 2;  // 16 KB: one [128 x 64] bf16 tile (Q, K or V)
 constexpr float ATT_RESCALE_LOG2 = 8.f;
 
 __device__ __forceinline__ float ex2(float x) {
@@ -30,273 +27,27 @@ __device__ __forceinline__ float ex2(float x) {
   return y;
 }
 
-template <bool V_KMAJOR>
-__global__ void __launch_bounds__(ATT_THREADS, 1)
-flash_attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                      const __grid_constant__ CUtensorMap tmV, int H, int N, float scale_log2, float scale,
-                      __nv_bfloat16* __restrict__ out, float* __restrict__ lse) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;
-  uint8_t* sK = sQ + ATT_TILE_BYTES;
-  uint8_t* sV = sK + ATT_KSTAGES * ATT_TILE_BYTES;
-  uint8_t* sP = sV + ATT_VSTAGES * ATT_TILE_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 2 * ATT_P_BYTES);
-  uint64_t* q_full = bars;                      // 1
-  uint64_t* k_full = q_full + 1;                // KSTAGES
-  uint64_t* k_empty = k_full + ATT_KSTAGES;     // KSTAGES
-  uint64_t* v_full = k_empty + ATT_KSTAGES;     // VSTAGES
-  uint64_t* v_empty = v_full + ATT_VSTAGES;     // VSTAGES
-  uint64_t* s_full = v_empty + ATT_VSTAGES;     // 2
-  uint64_t* s_free = s_full + 2;                // 2
-  uint64_t* p_full = s_free + 2;                // 2
-  uint64_t* pv_done = p_full + 2;               // 2
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(pv_done + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * ATT_BQ;
-  const int bh = blockIdx.y;
-  const int nkv = (N + ATT_BK - 1) / ATT_BK;
-
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK);
-    tma_prefetch_desc(&tmV);
-    mbar_init(smem_u32(q_full), 1);
-    for (int s = 0; s < ATT_KSTAGES; ++s) mbar_init(smem_u32(&k_full[s]), 1), mbar_init(smem_u32(&k_empty[s]), 1);
-    for (int s = 0; s < ATT_VSTAGES; ++s) mbar_init(smem_u32(&v_full[s]), 1), mbar_init(smem_u32(&v_empty[s]), 1);
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(smem_u32(&s_full[s]), 1);
-      mbar_init(smem_u32(&s_free[s]), 4);
-      mbar_init(smem_u32(&p_full[s]), 4);
-      mbar_init(smem_u32(&pv_done[s]), 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_O = tmem_base + 256;
-
-  if (warp == 0) {
-    if (lane == 0) {  // ===== TMA producer =====
-      mbar_expect_tx(smem_u32(q_full), ATT_TILE_BYTES);
-      tma_load_3d(smem_u32(sQ), &tmQ, smem_u32(q_full), 0, q0, bh);
-      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
-      for (int j = 0; j < nkv; ++j) {
-        mbar_wait(smem_u32(&k_empty[ks]), kph ^ 1);
-        mbar_expect_tx(smem_u32(&k_full[ks]), ATT_TILE_BYTES);
-        tma_load_3d(smem_u32(sK + ks * ATT_TILE_BYTES), &tmK, smem_u32(&k_full[ks]), 0, j * ATT_BK, bh);
-        if (++ks == ATT_KSTAGES) ks = 0, kph ^= 1;
-        mbar_wait(smem_u32(&v_empty[vs]), vph ^ 1);
-        mbar_expect_tx(smem_u32(&v_full[vs]), ATT_TILE_BYTES);
-        if (V_KMAJOR) {  // V^T [BH, 64, N]: two [64 d x 64 kv] boxes
-          tma_load_3d(smem_u32(sV + vs * ATT_TILE_BYTES), &tmV, smem_u32(&v_full[vs]), j * ATT_BK, 0, bh);
-          tma_load_3d(smem_u32(sV + vs * ATT_TILE_BYTES + ATT_TILE_BYTES / 2), &tmV, smem_u32(&v_full[vs]),
-                      j * ATT_BK + 64, 0, bh);
-        } else {  // V [BH, N, 64]: one [128 kv x 64 d] box
-          tma_load_3d(smem_u32(sV + vs * ATT_TILE_BYTES), &tmV, smem_u32(&v_full[vs]), 0, j * ATT_BK, bh);
-        }
-        if (++vs == ATT_VSTAGES) vs = 0, vph ^= 1;
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    if (lane == 0) {  // ===== MMA issuer =====
-      constexpr uint32_t idesc_s = umma_idesc(UMMA_BF16, 128, 128);
-      constexpr uint32_t idesc_o = umma_idesc(UMMA_BF16, 128, 64, 0, V_KMAJOR ? 0 : 1);
-      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
-      const uint32_t aQ = smem_u32(sQ);
-      auto issue_S = [&](int j) {
-        const uint32_t b = j & 1, u = j >> 1;
-        mbar_wait(smem_u32(&k_full[ks]), kph);
-        mbar_wait(smem_u32(&s_free[b]), (u & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t aK = smem_u32(sK + ks * ATT_TILE_BYTES);
-#pragma unroll
-        for (int k = 0; k < ATT_D / 16; ++k)
-          umma_f16_ss(tmem_base + b * 128, umma_desc(aQ + k * 32, 16, 1024, UMMA_SW_128B),
-                      umma_desc(aK + k * 32, 16, 1024, UMMA_SW_128B), idesc_s, k != 0);
-        umma_commit(smem_u32(&k_empty[ks]));
-        umma_commit(smem_u32(&s_full[b]));
-        if (++ks == ATT_KSTAGES) ks = 0, kph ^= 1;
-      };
-      mbar_wait(smem_u32(q_full), 0);
-      issue_S(0);
-      for (int j = 0; j < nkv; ++j) {
-        if (j + 1 < nkv) issue_S(j + 1);
-        const uint32_t b = j & 1;
-        mbar_wait(smem_u32(&p_full[b]), (j >> 1) & 1);
-        mbar_wait(smem_u32(&v_full[vs]), vph);
-        tc_fence_after();
-        const uint32_t aP = smem_u32(sP + b * ATT_P_BYTES);
-        const uint32_t aV = smem_u32(sV + vs * ATT_TILE_BYTES);
-#pragma unroll
-        for (int k = 0; k < ATT_BK / 16; ++k) {
-          const uint64_t pd = umma_desc(aP + (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32, 16, 1024, UMMA_SW_128B);
-          const uint64_t vd = V_KMAJOR
-                                  ? umma_desc(aV + (k >> 2) * (ATT_TILE_BYTES / 2) + (k & 3) * 32, 16, 1024, UMMA_SW_128B)
-                                  : umma_desc(aV + k * 2048, ATT_TILE_BYTES, 1024, UMMA_SW_128B);
-          umma_f16_ss(tmem_O, pd, vd, idesc_o, (j | k) != 0);
-        }
-        umma_commit(smem_u32(&v_empty[vs]));
-        umma_commit(smem_u32(&pv_done[b]));
-        if (++vs == ATT_VSTAGES) vs = 0, vph ^= 1;
-      }
-    }
-    __syncwarp();
-  } else if (warp >= 4) {  // ===== softmax: thread = query row =====
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-    float m_used = -INFINITY, l = 0.f;
-    for (int j = 0; j < nkv; ++j) {
-      const uint32_t b = j & 1, u = j >> 1;
-      mbar_wait(smem_u32(&s_full[b]), u & 1);
-      tc_fence_after();
-      uint32_t s[4][32];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) tmem_ld32(tmem_base + lane_base + b * 128 + c * 32, s[c]);
-      tmem_wait_ld();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&s_free[b]));
-      const int kv_valid = N - j * ATT_BK;  // >= 1
-      if (kv_valid < ATT_BK) {
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (c * 32 + i >= kv_valid) s[c][i] = __float_as_uint(-INFINITY);
-      }
-      float m_blk = -INFINITY;
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-#pragma unroll
-        for (int i = 0; i < 32; ++i) m_blk = fmaxf(m_blk, __uint_as_float(s[c][i]));
-      // P buffer b is free once PV(j-2) has retired
-      mbar_wait(smem_u32(&pv_done[b]), (u & 1) ^ 1);
-      bool need = false;
-      float alpha = 1.f;
-      if (j == 0) {
-        m_used = m_blk;
-      } else if ((m_blk - m_used) * scale_log2 > ATT_RESCALE_LOG2) {
-        need = true;
-        alpha = ex2((m_used - m_blk) * scale_log2);
-        m_used = m_blk;
-        l *= alpha;
-      }
-      if (__any_sync(0xffffffffu, need)) {  // rescale this warp's 32 rows of O in TMEM (rare after the first blocks)
-        mbar_wait(smem_u32(&pv_done[(j - 1) & 1]), ((j - 1) >> 1) & 1);
-        tc_fence_after();
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          uint32_t o[32];
-          tmem_ld32(tmem_O + lane_base + c * 32, o);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-          tmem_st32(tmem_O + lane_base + c * 32, o);
-        }
-        tmem_wait_st();
-      }
-      const float neg_m = -m_used * scale_log2;
-      uint8_t* prow = sP + b * ATT_P_BYTES + r * 128;
-      float sum = 0.f;
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint32_t pk[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          float p0 = ex2(fmaf(__uint_as_float(s[c][2 * i]), scale_log2, neg_m));
-          float p1 = ex2(fmaf(__uint_as_float(s[c][2 * i + 1]), scale_log2, neg_m));
-          sum += p0 + p1;
-          pk[i] = pack_bf16(p0, p1);
-        }
-        uint8_t* sub = prow + (c >> 1) * ATT_TILE_BYTES;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int chunk = ((c & 1) * 4 + i) ^ (r & 7);
-          *reinterpret_cast<uint4*>(sub + chunk * 16) = make_uint4(pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
-        }
-      }
-      l += sum;
-      fence_proxy_async_smem();  // P (generic-proxy stores) -> visible to the tensor core (async proxy)
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&p_full[b]));
-    }
-    // ---- epilogue: O / l -> bf16 [B, N, H*64] ----
-    mbar_wait(smem_u32(&pv_done[(nkv - 1) & 1]), ((nkv - 1) >> 1) & 1);
-    tc_fence_after();
-    const float inv_l = 1.f / l;
-    const int row = q0 + r;
-    const int bidx = bh / H, h = bh - bidx * H;
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      uint32_t o[32];
-      tmem_ld32(tmem_O + lane_base + c * 32, o);
-      tmem_wait_ld();
-      if (row < N) {
-        uint4* dst = reinterpret_cast<uint4*>(out + ((int64_t)bidx * N + row) * (H * ATT_D) + h * ATT_D + c * 32);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-          dst[i] = make_uint4(pack_bf16(__uint_as_float(o[8 * i]) * inv_l, __uint_as_float(o[8 * i + 1]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 2]) * inv_l, __uint_as_float(o[8 * i + 3]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 4]) * inv_l, __uint_as_float(o[8 * i + 5]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 6]) * inv_l, __uint_as_float(o[8 * i + 7]) * inv_l));
-      }
-    }
-    if (lse && row < N) lse[(int64_t)bh * N + row] = m_used * scale + logf(l);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_base, 512);
-}
-
-
-// =================================================================================================
-// v3 (default): two query tiles (256 rows) per CTA, two softmax warpgroups, everything but K/V/Q in TMEM.
-//   warpgroup 0 : warp 0 lane 0 = TMA producer, warp 1 / warp 2 lane 0 = MMA issuer of tile A / tile B
-//   warpgroup 1 : softmax of tile A (rows q0 .. q0+127), one row per thread;  warpgroup 2 : tile B
-//   TMEM        : S_A [0,128) S_B [128,256) | P_A [256,320) P_B [320,384) (bf16 pairs) | O_A [384,448) O_B [448,512)
-// The softmax releases S as soon as it sits in registers (s_free), so S(j+1) = Q K(j+1)^T is computed WHILE the
-// softmax of block j runs; P is written back to TMEM and feeds O += P V as the TMEM A operand (no smem round trip).
-// Each tile has its own issuing thread (blocking mbarrier waits in the tile's natural event order s_free, p_full, ...),
-// so neither tile queues behind the other's softmax.   Packed f32x2 math (FFMA2/FADD2) + FMNMX3.
-// =================================================================================================
 constexpr int A2_THREADS = 384;
 constexpr int A2_KSTAGES = 4, A2_VSTAGES = 4;
-constexpr int A2_SMEM = ATT_TILE_BYTES * (2 + A2_KSTAGES + A2_VSTAGES) + 3 * 128 * 32 + 1024 + 256;
+constexpr int A2_SMEM = ATT_TILE_BYTES * (2 + A2_KSTAGES + A2_VSTAGES) + 1024 + 256;
 
-#ifdef SMBV_DEV_BUILD
-// developer timeline trace (stagger_ns == -1): clock64 of one CTA's softmax warps at the main hand-offs, [event + 6*tile][block]
-__device__ long long g_ftrace[12][32];
-#endif
+// Pair i of every 16-pair chunk of exponentials runs as ex2_emu2 on the FMA / ALU pipes when bit i is set, else on MUFU.EX2.
+// 6 of every 16 pairs (37.5 %): measured on one box, same run: 1.52 ms vs 1.60 ms all-MUFU at H=12, N=20480 (-5 %; also -5 % at
+// H=6 and at N=7168); 25 % and 31 % gain less, 44 % and 50 % fall off a cliff (1.78 / 1.85 ms: the softmax warps become
+// issue-bound), other placements of the six pairs are 1-7 % slower.
+constexpr uint32_t EX2_EMU_PAIRS = 0xA4A4u;
 
-// FOLD (experiment, `make DEV=1` + SMBV_ATTN_FOLD=1; measured NEUTRAL in round 2, see profiles/r02_attn_notes.md): the per-element `x = s * scale_log2 - m * scale_log2` (one packed FFMA2 per pair: 16 % of the FP32 / ALU pipe
-// work that bounds this kernel — profiles/r02_attn_notes.md) is moved into the tensor core.  The softmax warpgroup multiplies its Q
-// tile by scale * log2(e) once (in shared memory, fp32 multiply, bf16 store), and the score MMA gets a FIFTH K-step whose operands
-// are a [128 x 16] tile holding -m (the running row maximum in log2 units, kept bf16-representable) in its first column and a
-// constant [128 x 16] tile with 1 in its first column: the tile that comes back already holds x = q'.k - m.  A thread rewrites
-// its -m only when the block maximum exceeds the running one by more than 2^8 (and in the first block) — such a block takes
-// the path with the extra subtraction — and always BEFORE it releases S for the next score MMA.
-constexpr int A2_EXT_BYTES = 128 * 32;  // [128 rows x 16 bf16], K-major, no swizzle: (r / 8) * 256 + (k / 8) * 128 + (r % 8) * 16 + (k % 8) * 2
-template <uint32_t EMU_MASK, bool FOLD = false>  // EMU_MASK bit i: pair i of every 16-pair chunk uses ex2_emu2 instead of MUFU.EX2
 __global__ void __launch_bounds__(A2_THREADS, 1)
 flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                        const __grid_constant__ CUtensorMap tmV, int H, int N, float scale_log2, float scale,
                        __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int n_full, int n_split, int parts, int pairs_per_head,
-                       float* __restrict__ ws, int stagger_ns) {
+                       float* __restrict__ ws) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;  // 2 tiles
   uint8_t* sK = sQ + 2 * ATT_TILE_BYTES;
   uint8_t* sV = sK + A2_KSTAGES * ATT_TILE_BYTES;
-  uint8_t* sX = sV + A2_VSTAGES * ATT_TILE_BYTES;  // FOLD: [-m | 0...] of tile A, of tile B, then the constant [1 | 0...] tile
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sX + 3 * A2_EXT_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + A2_VSTAGES * ATT_TILE_BYTES);
   uint64_t* q_full = bars;
   uint64_t* k_full = q_full + 1;
   uint64_t* k_empty = k_full + A2_KSTAGES;
@@ -380,9 +131,6 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       const uint64_t dQ = umma_desc(smem_u32(sQ + t * ATT_TILE_BYTES), 16, 1024, UMMA_SW_128B);
       const uint64_t dK = umma_desc(smem_u32(sK), 16, 1024, UMMA_SW_128B);
       const uint64_t dV = umma_desc(smem_u32(sV), ATT_TILE_BYTES, 1024, UMMA_SW_128B);
-      // no-swizzle K-major [128 x 16] tiles: LBO = 128 B between the two 8-element core matrices along K, SBO = 256 B between 8-row groups
-      const uint64_t dQx = umma_desc(smem_u32(sX + t * A2_EXT_BYTES), 128, 256, UMMA_SW_NONE);  // (validated on B200: the swapped roles give garbage)
-      const uint64_t dKx = umma_desc(smem_u32(sX + 2 * A2_EXT_BYTES), 128, 256, UMMA_SW_NONE);
       const uint32_t tS = tmem_base + t * 128, tP = tmem_base + 256 + t * 64, tO = tmem_base + 384 + t * 64;
       uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
       auto issue_S = [&]() {  // S_t = Q_t K(stage ks)^T, then release the K stage (both issuers arrive on k_empty)
@@ -391,22 +139,15 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
         const uint64_t b = dK + (uint64_t)((ks * ATT_TILE_BYTES) >> 4);
 #pragma unroll
         for (int k = 0; k < ATT_D / 16; ++k) umma_f16_ss(tS, dQ + 2 * k, b + 2 * k, idesc_s, k != 0);
-        if (FOLD) umma_f16_ss(tS, dQx, dKx, idesc_s, 1);  // fifth K-step: + (-m) * 1
         umma_commit(smem_u32(&s_full[t]));
         umma_commit(smem_u32(&k_empty[ks]));
         if (++ks == A2_KSTAGES) ks = 0, kph ^= 1;
       };
-      if (FOLD) {  // the softmax warpgroup has scaled Q in shared memory and zero-filled the S columns (first s_free phase)
-        mbar_wait(smem_u32(&s_free[t]), 0);
-        tc_fence_after();
-      } else {
-        mbar_wait(smem_u32(q_full), 0);
-      }
+      mbar_wait(smem_u32(q_full), 0);
       issue_S();
       for (int j = 0; j < nkv; ++j) {
         if (j + 1 < nkv) {  // S(j+1) as soon as the softmax has pulled S(j) into registers: runs under softmax(j)
-          mbar_wait(smem_u32(&s_free[t]), FOLD ? ((j + 1) & 1) : (j & 1));
-          if (FOLD) tc_fence_after();
+          mbar_wait(smem_u32(&s_free[t]), j & 1);
           issue_S();
         }
         mbar_wait(smem_u32(&v_full[vs]), vph);
@@ -432,57 +173,21 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     const uint32_t tP = tmem_base + lane_base + 256 + t * 64;
     const uint32_t tO = tmem_base + lane_base + 384 + t * 64;
     const uint64_t sc2 = pack2(scale_log2, scale_log2);
-    float m_used = FOLD ? 0.f : -INFINITY, l = 0.f;  // FOLD: log2 units, and what the score MMA currently subtracts (0 at first)
+    float m_used = -INFINITY, l = 0.f;
     // barrier addresses as 32-bit shared-window offsets held in registers of THIS register region: the generic `bars`
     // pointer lives across the setmaxnreg boundary and was re-loaded from local memory (LDL) in front of every arrive / wait
     uint32_t b_sfull = smem_u32(&s_full[t]), b_sfree = smem_u32(&s_free[t]), b_pfull = smem_u32(&p_full[t]), b_pvdone = smem_u32(&pv_done[t]);
     asm volatile("" : "+r"(b_sfull), "+r"(b_sfree), "+r"(b_pfull), "+r"(b_pvdone));
-#ifdef SMBV_DEV_BUILD
-    const bool tr = stagger_ns == -1 && blockIdx.x == 5 && lane == 0 && quad == 0;
-#define SMBV_FTR(ev) do { if (tr && j >= 8 && j < 40) g_ftrace[(ev) + 6 * t][j - 8] = clock64(); } while (0)
-#else
-#define SMBV_FTR(ev) do { } while (0)
-#endif
-    if (FOLD) {  // ---- Q_t *= scale * log2(e) in shared memory (row r of the tile; element-wise, so the 128B swizzle does not matter) ----
-      mbar_wait(smem_u32(q_full), 0);
-      uint4* qrow = reinterpret_cast<uint4*>(sQ + t * ATT_TILE_BYTES + r * 128);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        uint4 v = qrow[i];
-        uint32_t* w = reinterpret_cast<uint32_t*>(&v);
-#pragma unroll
-        for (int e = 0; e < 4; ++e)
-          w[e] = pack_bf16(__uint_as_float(w[e] << 16) * scale_log2, __uint_as_float(w[e] & 0xFFFF0000u) * scale_log2);
-        qrow[i] = v;
-      }
-      // row r of this tile's [-m | 0...] operand (m = 0 for the first block) and of the constant [1 | 0...] one
-      uint4* xr = reinterpret_cast<uint4*>(sX + t * A2_EXT_BYTES + (r >> 3) * 256 + (r & 7) * 16);
-      xr[0] = make_uint4(0u, 0u, 0u, 0u), xr[8] = make_uint4(0u, 0u, 0u, 0u);  // k 0..7 and (128 B further) k 8..15
-      if (t == 0) {
-        uint4* kr = reinterpret_cast<uint4*>(sX + 2 * A2_EXT_BYTES + (r >> 3) * 256 + (r & 7) * 16);
-        kr[0] = make_uint4(0x3F80u, 0u, 0u, 0u), kr[8] = make_uint4(0u, 0u, 0u, 0u);  // bf16 1.0 in column 0
-      }
-      fence_proxy_async_smem();  // generic-proxy stores -> visible to the tensor core's (async proxy) operand reads
-      __syncwarp();
-      if (lane == 0) mbar_arrive(b_sfree);
-    }
     for (int j = 0; j < nkv; ++j) {
       mbar_wait(b_sfull, j & 1);
-      SMBV_FTR(0);
-#ifdef SMBV_DEV_BUILD
-      if (j == 0 && t == 1 && stagger_ns > 0) __nanosleep(stagger_ns);
-#endif
       tc_fence_after();
       uint32_t s[4][32];
 #pragma unroll
       for (int c = 0; c < 4; ++c) tmem_ld32(tS + c * 32, s[c]);
       tmem_wait_ld();
-      SMBV_FTR(1);
-      if (!FOLD) {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(b_sfree);  // S(j+1) may now overwrite the S columns
-      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(b_sfree);  // S(j+1) may now overwrite the S columns
       const int kv_valid = N - (kv_begin + j) * ATT_BK;
       if (kv_valid < ATT_BK) {
 #pragma unroll
@@ -507,104 +212,44 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       float alpha = 1.f;
       uint64_t acc[4] = {0ull, 0ull, 0ull, 0ull};
       uint32_t pk[4][16];
-      if (FOLD) {
-        // s[] already holds x' = q'.k - m_used (log2 units; m_used = 0 in the first block).  delta = what still has to come off.
-        float delta = 0.f;
-        if (j == 0 || m_blk > ATT_RESCALE_LOG2) {
-          // new running maximum, rounded UP to a bf16-representable value (it is an operand of the score MMA from now on)
-          const uint32_t mb = __float_as_uint(m_used + m_blk);
-          const float m_new = __uint_as_float((mb & 0x80000000u) ? (mb & 0xFFFF0000u) : ((mb + 0xFFFFu) & 0xFFFF0000u));
-          delta = m_new - m_used;  // exact: both are bf16 values of similar magnitude ... or m_used == 0
-          m_used = m_new;
-          if (j > 0) {
-            need = true;
-            alpha = ex2(-delta);
-            l *= alpha;
+      auto chunk = [&](int c, uint64_t nm2, uint64_t (&a4)[4]) {  // 32 columns: p = 2^(s * scale_log2 + nm), packed bf16 + row-sum terms
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const uint64_t x2 = ffma2(pack2(__uint_as_float(s[c][2 * i]), __uint_as_float(s[c][2 * i + 1])), sc2, nm2);
+          float p0, p1;
+          if ((EX2_EMU_PAIRS >> i) & 1u) {
+            ex2_emu2(x2, p0, p1);
+          } else {
+            float a, b;
+            unpack2(x2, a, b);
+            p0 = ex2(a), p1 = ex2(b);
           }
-          *reinterpret_cast<uint16_t*>(sX + t * A2_EXT_BYTES + (r >> 3) * 256 + (r & 7) * 16) = (uint16_t)(__float_as_uint(-m_new) >> 16);
-          fence_proxy_async_smem();
+          a4[i & 3] = fadd2(a4[i & 3], pack2(p0, p1));
+          pk[c][i] = pack_bf16(p0, p1);
         }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(b_sfree);  // S(j+1) may now overwrite the S columns (and reads the -m just written)
-        const bool slow = __any_sync(0xffffffffu, delta != 0.f);  // first block, or the running maximum moved: rare afterwards
-        if (slow) {
-          const uint64_t nd2 = pack2(-delta, -delta);
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const uint64_t x2 = fadd2(pack2(__uint_as_float(s[c][2 * i]), __uint_as_float(s[c][2 * i + 1])), nd2);
-              float p0, p1;
-              if ((EMU_MASK >> i) & 1u) {
-                ex2_emu2(x2, p0, p1);
-              } else {
-                float a, b;
-                unpack2(x2, a, b);
-                p0 = ex2(a), p1 = ex2(b);
-              }
-              acc[i & 3] = fadd2(acc[i & 3], pack2(p0, p1));
-              pk[c][i] = pack_bf16(p0, p1);
-            }
-          }
-        } else {
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              float p0, p1;
-              if ((EMU_MASK >> i) & 1u) {
-                ex2_emu2(pack2(__uint_as_float(s[c][2 * i]), __uint_as_float(s[c][2 * i + 1])), p0, p1);
-              } else {
-                p0 = ex2(__uint_as_float(s[c][2 * i])), p1 = ex2(__uint_as_float(s[c][2 * i + 1]));
-              }
-              acc[i & 3] = fadd2(acc[i & 3], pack2(p0, p1));
-              pk[c][i] = pack_bf16(p0, p1);
-            }
-          }
-        }
-      } else {
-        auto chunk = [&](int c, uint64_t nm2, uint64_t (&a4)[4]) {  // 32 columns: p = 2^(s * scale_log2 + nm), packed bf16 + row-sum terms
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            const uint64_t x2 = ffma2(pack2(__uint_as_float(s[c][2 * i]), __uint_as_float(s[c][2 * i + 1])), sc2, nm2);
-            float p0, p1;
-            if ((EMU_MASK >> i) & 1u) {
-              ex2_emu2(x2, p0, p1);
-            } else {
-              float a, b;
-              unpack2(x2, a, b);
-              p0 = ex2(a), p1 = ex2(b);
-            }
-            a4[i & 3] = fadd2(a4[i & 3], pack2(p0, p1));
-            pk[c][i] = pack_bf16(p0, p1);
-          }
-        };
-        if (j == 0) {
-          m_used = m_blk;
-        } else if ((m_blk - m_used) * scale_log2 > ATT_RESCALE_LOG2) {
-          need = true;
-          alpha = ex2((m_used - m_blk) * scale_log2);
-          m_used = m_blk;
-          l *= alpha;
-        }
-        const float nm = -m_used * scale_log2;
-        const uint64_t nm2 = pack2(nm, nm);
-#pragma unroll
-        for (int c = 0; c < 4; ++c) chunk(c, nm2, acc);
+      };
+      if (j == 0) {
+        m_used = m_blk;
+      } else if ((m_blk - m_used) * scale_log2 > ATT_RESCALE_LOG2) {
+        need = true;
+        alpha = ex2((m_used - m_blk) * scale_log2);
+        m_used = m_blk;
+        l *= alpha;
       }
+      const float nm = -m_used * scale_log2;
+      const uint64_t nm2 = pack2(nm, nm);
+#pragma unroll
+      for (int c = 0; c < 4; ++c) chunk(c, nm2, acc);
       {
         float a0, a1, b0, b1, c0, c1, d0, d1;
         unpack2(acc[0], a0, a1), unpack2(acc[1], b0, b1), unpack2(acc[2], c0, c1), unpack2(acc[3], d0, d1);
         l += ((a0 + a1) + (b0 + b1)) + ((c0 + c1) + (d0 + d1));
       }
-      SMBV_FTR(2);
       // PV(j-1) must have retired before P is overwritten / O is rescaled; by now it has had a whole softmax to do so
       if (j > 0) {
         mbar_wait(b_pvdone, (j - 1) & 1);
         tc_fence_after();
       }
-      SMBV_FTR(3);
       if (__any_sync(0xffffffffu, need)) {
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
@@ -619,12 +264,10 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
 #pragma unroll
       for (int c = 0; c < 4; ++c) tmem_st16(tP + c * 16, pk[c]);
       tmem_wait_st();
-      SMBV_FTR(4);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(b_pfull);
     }
-#undef SMBV_FTR
     mbar_wait(b_pvdone, (nkv - 1) & 1);
     tc_fence_after();
     const float inv_l = 1.f / l;
@@ -642,7 +285,7 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           *reinterpret_cast<float4*>(wo + c * 32 + 4 * i) = make_float4(__uint_as_float(o[4 * i]), __uint_as_float(o[4 * i + 1]),
                                                                          __uint_as_float(o[4 * i + 2]), __uint_as_float(o[4 * i + 3]));
       }
-      wo[64] = FOLD ? m_used * 0.69314718056f : m_used * scale;  // natural-log units (FOLD keeps the maximum in log2 units)
+      wo[64] = m_used * scale;  // natural-log units
       wo[65] = l;
     } else {
 #pragma unroll
@@ -660,304 +303,13 @@ flash_attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
                               pack_bf16(__uint_as_float(o[8 * i + 6]) * inv_l, __uint_as_float(o[8 * i + 7]) * inv_l));
       }
     }
-    if (lse && row < N) lse[(int64_t)bh * N + row] = (FOLD ? m_used * 0.69314718056f : m_used * scale) + logf(l);
+    if (lse && row < N) lse[(int64_t)bh * N + row] = m_used * scale + logf(l);
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, 512);
 }
-
-#ifdef SMBV_DEV_BUILD  // experiment kept for the record (profiles/r01_attn_notes.md); not in the release library
-// =================================================================================================
-// v4: the same CTA (two query tiles, TMEM layout, MMA issuers) with FOUR softmax warpgroups: each tile's 128 score columns
-// are split between two warpgroups (64 columns per thread).  Timeline traces of v3 (tools/trace_attn_fwd.py) show one softmax
-// warp per tile per scheduler leaving the MUFU pipe idle ~19 % of the time (a lone warp in its exp phase does not saturate
-// it with this instruction mix, and the load / max / store phases of the two tiles overlap too little); with two warps per
-// tile per scheduler the pipe always has ready work.  The two halves of a row agree on the block maximum through a
-// double-buffered shared-memory exchange + one named barrier per tile and block; row sums stay partial until the end.
-// =================================================================================================
-constexpr int A4_THREADS = 640;
-constexpr int A4_SMEM = A2_SMEM + 1024 + 2 * 2 * 2 * 128 * 4;  // + max exchange [parity][tile][half][row]
-
-template <uint32_t EMU4>
-__global__ void __launch_bounds__(A4_THREADS, 1)
-flash_attn_fwd4_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                       const __grid_constant__ CUtensorMap tmV, int H, int N, float scale_log2, float scale,
-                       __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int n_full, int n_split, int parts, int pairs_per_head,
-                       float* __restrict__ ws) {
-  constexpr bool FOLD = false;     // (the fifth-K-step experiment exists only in the two-warpgroup kernel)
-  const uint64_t dQx = 0, dKx = 0;
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;  // 2 tiles
-  uint8_t* sK = sQ + 2 * ATT_TILE_BYTES;
-  uint8_t* sV = sK + A2_KSTAGES * ATT_TILE_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + A2_VSTAGES * ATT_TILE_BYTES);
-  uint64_t* q_full = bars;
-  uint64_t* k_full = q_full + 1;
-  uint64_t* k_empty = k_full + A2_KSTAGES;
-  uint64_t* v_full = k_empty + A2_KSTAGES;
-  uint64_t* v_empty = v_full + A2_VSTAGES;
-  uint64_t* s_full = v_empty + A2_VSTAGES;  // [2] per tile
-  uint64_t* s_free = s_full + 2;            // [2]
-  uint64_t* p_full = s_free + 2;            // [2]
-  uint64_t* pv_done = p_full + 2;           // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(pv_done + 2);
-  float* xm = reinterpret_cast<float*>(smem + A2_SMEM - 1024 - 256 + 1024);  // after the barrier block (which is < 1 KB)
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // Work decomposition.  A unit = a PAIR of adjacent 128-row query tiles of one head (the ping-pong mode).  The first
-  // n_full CTAs run whole units.  The units that would form a last, partial wave are each split over `parts` CTAs by key
-  // range (wave-quantisation fix: the tail then costs 1/parts .. of a CTA time); those CTAs leave un-normalised partial results
-  // (O, max, sum) in `ws` and flash_attn_combine_kernel merges the halves.  A head with an odd number of tiles ends with
-  // one single-tile CTA.
-  int q0, bh, ntiles = 2, kv_begin = 0, split_slot = -1;
-  const int nkv_total = (N + ATT_BK - 1) / ATT_BK;
-  int nkv = nkv_total;
-  {
-    const int b = blockIdx.x;
-    if (b < n_full) {
-      bh = b / pairs_per_head, q0 = 2 * (b % pairs_per_head) * ATT_BQ;
-    } else if (b < n_full + parts * n_split) {
-      const int s1 = b - n_full, pr = n_full + s1 / parts, part = s1 % parts;
-      bh = pr / pairs_per_head, q0 = 2 * (pr % pairs_per_head) * ATT_BQ;
-      kv_begin = (int)((int64_t)nkv_total * part / parts);
-      nkv = (int)((int64_t)nkv_total * (part + 1) / parts) - kv_begin;
-      split_slot = s1;  // (unit, part)
-    } else {  // odd leftover tile of a head
-      bh = b - n_full - parts * n_split, q0 = ((N + ATT_BQ - 1) / ATT_BQ - 1) * ATT_BQ, ntiles = 1;
-    }
-  }
-
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK);
-    tma_prefetch_desc(&tmV);
-    mbar_init(smem_u32(q_full), 1);
-    for (int s = 0; s < A2_KSTAGES; ++s) mbar_init(smem_u32(&k_full[s]), 1), mbar_init(smem_u32(&k_empty[s]), ntiles);
-    for (int s = 0; s < A2_VSTAGES; ++s) mbar_init(smem_u32(&v_full[s]), 1), mbar_init(smem_u32(&v_empty[s]), ntiles);
-    for (int t = 0; t < 2; ++t) {
-      mbar_init(smem_u32(&s_full[t]), 1);
-      mbar_init(smem_u32(&s_free[t]), 8);  // two warpgroups per tile
-      mbar_init(smem_u32(&p_full[t]), 8);
-      mbar_init(smem_u32(&pv_done[t]), 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < 4) {
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
-    if (warp == 0 && lane == 0) {  // ===== TMA producer =====
-      mbar_expect_tx(smem_u32(q_full), ntiles * ATT_TILE_BYTES);
-      tma_load_3d(smem_u32(sQ), &tmQ, smem_u32(q_full), 0, q0, bh);
-      if (ntiles == 2) tma_load_3d(smem_u32(sQ + ATT_TILE_BYTES), &tmQ, smem_u32(q_full), 0, q0 + ATT_BQ, bh);
-      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
-      for (int j = 0; j < nkv; ++j) {
-        mbar_wait(smem_u32(&k_empty[ks]), kph ^ 1);
-        mbar_expect_tx(smem_u32(&k_full[ks]), ATT_TILE_BYTES);
-        tma_load_3d(smem_u32(sK + ks * ATT_TILE_BYTES), &tmK, smem_u32(&k_full[ks]), 0, (kv_begin + j) * ATT_BK, bh);
-        if (++ks == A2_KSTAGES) ks = 0, kph ^= 1;
-        mbar_wait(smem_u32(&v_empty[vs]), vph ^ 1);
-        mbar_expect_tx(smem_u32(&v_full[vs]), ATT_TILE_BYTES);
-        tma_load_3d(smem_u32(sV + vs * ATT_TILE_BYTES), &tmV, smem_u32(&v_full[vs]), 0, (kv_begin + j) * ATT_BK, bh);
-        if (++vs == A2_VSTAGES) vs = 0, vph ^= 1;
-      }
-    } else if ((warp == 1 || (warp == 2 && ntiles == 2)) && elect_one()) {  // ===== MMA issuers: warp 1 -> tile A, warp 2 -> tile B =====
-      // elect.sync, not `lane == 0`: with a threadIdx-derived predicate ptxas cannot prove a single active lane and wraps every
-      // tcgen05.mma in an ELECT / R2UR / BRA.U.ANY waterfall loop (~75 cycles of issue per MMA, 12 MMAs per score tile)
-      const int t = warp - 1;
-      constexpr uint32_t idesc_s = umma_idesc(UMMA_BF16, 128, 128);
-      constexpr uint32_t idesc_o = umma_idesc(UMMA_BF16, 128, 64, 0, 1);  // V is the MN-major B operand
-      // descriptor templates: only the 14-bit start-address field changes (+ bytes >> 4)
-      const uint64_t dQ = umma_desc(smem_u32(sQ + t * ATT_TILE_BYTES), 16, 1024, UMMA_SW_128B);
-      const uint64_t dK = umma_desc(smem_u32(sK), 16, 1024, UMMA_SW_128B);
-      const uint64_t dV = umma_desc(smem_u32(sV), ATT_TILE_BYTES, 1024, UMMA_SW_128B);
-      const uint32_t tS = tmem_base + t * 128, tP = tmem_base + 256 + t * 64, tO = tmem_base + 384 + t * 64;
-      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
-      auto issue_S = [&]() {  // S_t = Q_t K(stage ks)^T, then release the K stage (both issuers arrive on k_empty)
-        mbar_wait(smem_u32(&k_full[ks]), kph);
-        tc_fence_after();
-        const uint64_t b = dK + (uint64_t)((ks * ATT_TILE_BYTES) >> 4);
-#pragma unroll
-        for (int k = 0; k < ATT_D / 16; ++k) umma_f16_ss(tS, dQ + 2 * k, b + 2 * k, idesc_s, k != 0);
-        if (FOLD) umma_f16_ss(tS, dQx, dKx, idesc_s, 1);  // fifth K-step: + (-m) * 1
-        umma_commit(smem_u32(&s_full[t]));
-        umma_commit(smem_u32(&k_empty[ks]));
-        if (++ks == A2_KSTAGES) ks = 0, kph ^= 1;
-      };
-      if (FOLD) {  // the softmax warpgroup has scaled Q in shared memory and zero-filled the S columns (first s_free phase)
-        mbar_wait(smem_u32(&s_free[t]), 0);
-        tc_fence_after();
-      } else {
-        mbar_wait(smem_u32(q_full), 0);
-      }
-      issue_S();
-      for (int j = 0; j < nkv; ++j) {
-        if (j + 1 < nkv) {  // S(j+1) as soon as the softmax has pulled S(j) into registers: runs under softmax(j)
-          mbar_wait(smem_u32(&s_free[t]), FOLD ? ((j + 1) & 1) : (j & 1));
-          if (FOLD) tc_fence_after();
-          issue_S();
-        }
-        mbar_wait(smem_u32(&v_full[vs]), vph);
-        mbar_wait(smem_u32(&p_full[t]), j & 1);
-        tc_fence_after();
-        const uint64_t b = dV + (uint64_t)((vs * ATT_TILE_BYTES) >> 4);
-#pragma unroll
-        for (int k = 0; k < ATT_BK / 16; ++k)  // A = P[128 x 16] as bf16 pairs in 8 TMEM columns
-          umma_f16_ts(tO, tP + k * 8, b + (uint64_t)(k * 128), idesc_o, (j | k) != 0);
-        umma_commit(smem_u32(&pv_done[t]));
-        umma_commit(smem_u32(&v_empty[vs]));
-        if (++vs == A2_VSTAGES) vs = 0, vph ^= 1;
-      }
-    }
-    __syncwarp();
-  } else if (((warp >> 2) - 1) >> 1 < ntiles) {  // ===== softmax: warpgroup g -> tile g/2, score columns [64 (g&1), +64) =====
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 104;");
-    const int g = (warp >> 2) - 1;
-    const int t = g >> 1, hf = g & 1;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-    const uint32_t tS = tmem_base + lane_base + t * 128 + hf * 64;
-    const uint32_t tP = tmem_base + lane_base + 256 + t * 64 + hf * 32;
-    const uint32_t tO = tmem_base + lane_base + 384 + t * 64 + hf * 32;
-    const uint64_t sc2 = pack2(scale_log2, scale_log2);
-    float m_used = -INFINITY, l = 0.f;
-    for (int j = 0; j < nkv; ++j) {
-      mbar_wait(smem_u32(&s_full[t]), j & 1);
-      tc_fence_after();
-      uint32_t s[2][32];
-      tmem_ld32(tS, s[0]);
-      tmem_ld32(tS + 32, s[1]);
-      tmem_wait_ld();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&s_free[t]));  // S(j+1) may now overwrite the S columns
-      const int kv_valid = N - (kv_begin + j) * ATT_BK - hf * 64;
-      if (kv_valid < 64) {
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (c * 32 + i >= kv_valid) s[c][i] = __float_as_uint(-INFINITY);
-      }
-      float mx[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-      for (int c = 0; c < 2; ++c)
-#pragma unroll
-        for (int i = 0; i < 32; i += 8) {
-          mx[0] = fmax3(mx[0], __uint_as_float(s[c][i]), __uint_as_float(s[c][i + 1]));
-          mx[1] = fmax3(mx[1], __uint_as_float(s[c][i + 2]), __uint_as_float(s[c][i + 3]));
-          mx[2] = fmax3(mx[2], __uint_as_float(s[c][i + 4]), __uint_as_float(s[c][i + 5]));
-          mx[3] = fmax3(mx[3], __uint_as_float(s[c][i + 6]), __uint_as_float(s[c][i + 7]));
-        }
-      float m_blk = fmaxf(fmaxf(mx[0], mx[1]), fmaxf(mx[2], mx[3]));
-      {  // agree on the row maximum with the thread that holds the other 64 columns of this row
-        float* slot = xm + (((j & 1) * 2 + t) * 2) * 128;
-        slot[hf * 128 + r] = m_blk;
-        asm volatile("bar.sync %0, 256;" ::"r"(1 + t) : "memory");
-        m_blk = fmaxf(m_blk, slot[(hf ^ 1) * 128 + r]);
-      }
-      bool need = false;
-      float alpha = 1.f;
-      if (j == 0) {
-        m_used = m_blk;
-      } else if ((m_blk - m_used) * scale_log2 > ATT_RESCALE_LOG2) {
-        need = true;
-        alpha = ex2((m_used - m_blk) * scale_log2);
-        m_used = m_blk;
-        l *= alpha;
-      }
-      // PV(j-1) must have retired before P is overwritten / O is rescaled (it was issued a whole softmax ago)
-      if (j > 0) {
-        mbar_wait(smem_u32(&pv_done[t]), (j - 1) & 1);
-        tc_fence_after();
-      }
-      if (__any_sync(0xffffffffu, need)) {  // this warpgroup's 32 of the 64 O columns
-        uint32_t o[32];
-        tmem_ld32(tO, o);
-        tmem_wait_ld();
-#pragma unroll
-        for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-        tmem_st32(tO, o);
-      }
-      const float nm = -m_used * scale_log2;
-      const uint64_t nm2 = pack2(nm, nm);
-      uint64_t acc[2] = {0ull, 0ull};
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        uint32_t pk[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const uint64_t x2 = ffma2(pack2(__uint_as_float(s[c][2 * i]), __uint_as_float(s[c][2 * i + 1])), sc2, nm2);
-          float p0, p1;
-          if ((EMU4 >> i) & 1u) {
-            ex2_emu2(x2, p0, p1);
-          } else {
-            float a, b;
-            unpack2(x2, a, b);
-            p0 = ex2(a), p1 = ex2(b);
-          }
-          acc[i & 1] = fadd2(acc[i & 1], pack2(p0, p1));
-          pk[i] = pack_bf16(p0, p1);
-        }
-        tmem_st16(tP + c * 16, pk);  // P goes out chunk by chunk: 16 live registers instead of 32
-      }
-      {
-        float a0, a1, b0, b1;
-        unpack2(acc[0], a0, a1), unpack2(acc[1], b0, b1);
-        l += (a0 + a1) + (b0 + b1);
-      }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&p_full[t]));
-    }
-    mbar_wait(smem_u32(&pv_done[t]), (nkv - 1) & 1);
-    tc_fence_after();
-    {  // total row sum = the two halves' partial sums (same m_used on both sides by construction)
-      float* slot = xm + (((nkv & 1) * 2 + t) * 2) * 128;
-      slot[hf * 128 + r] = l;
-      asm volatile("bar.sync %0, 256;" ::"r"(1 + t) : "memory");
-      l += slot[(hf ^ 1) * 128 + r];
-    }
-    const float inv_l = 1.f / l;
-    const int row = q0 + t * ATT_BQ + r;
-    const int bidx = bh / H, h = bh - bidx * H;
-    uint32_t o[32];
-    tmem_ld32(tO, o);
-    tmem_wait_ld();
-    if (split_slot >= 0) {  // key-range half of a split unit: leave (O un-normalised, max, sum) for the combine kernel
-      float* wo = ws + ((int64_t)(split_slot * 2 + t) * ATT_BQ + r) * 68;
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-        *reinterpret_cast<float4*>(wo + hf * 32 + 4 * i) = make_float4(__uint_as_float(o[4 * i]), __uint_as_float(o[4 * i + 1]),
-                                                                          __uint_as_float(o[4 * i + 2]), __uint_as_float(o[4 * i + 3]));
-      if (hf == 0) wo[64] = m_used * scale, wo[65] = l;  // natural-log units
-    } else {
-      if (row < N) {
-        uint4* dst = reinterpret_cast<uint4*>(out + ((int64_t)bidx * N + row) * (H * ATT_D) + h * ATT_D + hf * 32);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-          dst[i] = make_uint4(pack_bf16(__uint_as_float(o[8 * i]) * inv_l, __uint_as_float(o[8 * i + 1]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 2]) * inv_l, __uint_as_float(o[8 * i + 3]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 4]) * inv_l, __uint_as_float(o[8 * i + 5]) * inv_l),
-                              pack_bf16(__uint_as_float(o[8 * i + 6]) * inv_l, __uint_as_float(o[8 * i + 7]) * inv_l));
-        if (lse && hf == 0) lse[(int64_t)bh * N + row] = m_used * scale + logf(l);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_base, 512);
-}
-#endif  // SMBV_DEV_BUILD
 
 // merges the `parts` key-range pieces of every split unit: one warp per query row, 2 columns per lane
 __global__ void __launch_bounds__(256) flash_attn_combine_kernel(const float* __restrict__ ws, int n_full, int n_split, int parts,
@@ -996,7 +348,6 @@ static int attn_tmap(CUtensorMap* m, const void* base, int BH, int N, int box_ro
 
 using namespace smbv;
 
-// v_kmajor: 0 = v2 kernel, V [BH,N,64];  1 = v1 kernel with V^T [BH,64,N] (N % 8 == 0);  2 = v1 kernel, V [BH,N,64]
 // split of the partial last wave: `rest` units cut into `parts` key ranges each (0 = no split).  Cost of the tail in units of one
 // whole CTA: rounds(k) * (1/k + fixed/nkv), fixed = the per-CTA prologue + epilogue in key-block times (Q load, TMEM allocation,
 // pipeline fill, O write-back ~ 3 blocks): short units (1960 tokens = 16 blocks) must not be cut into 3-block pieces
@@ -1021,7 +372,7 @@ extern "C" int64_t smbv_flash_attn_fwd_workspace_bytes(int B, int H, int N) {
 }
 
 extern "C" int smbv_flash_attn_fwd_ex(const smbv_bf16* q, const smbv_bf16* k, const smbv_bf16* v, int B, int H, int N,
-                                      float scale, smbv_bf16* out, float* lse, int v_kmajor, void* workspace,
+                                      float scale, smbv_bf16* out, float* lse, int variant, void* workspace,
                                       int64_t workspace_bytes, smbv_stream_t st) {
   SMBV_ARG(q && k && v && out, "flash_attn_fwd: null pointer");
   SMBV_ARG(B > 0 && H > 0 && N > 0, "flash_attn_fwd: bad sizes B=%d H=%d N=%d", B, H, N);
@@ -1029,111 +380,40 @@ extern "C" int smbv_flash_attn_fwd_ex(const smbv_bf16* q, const smbv_bf16* k, co
              reinterpret_cast<uintptr_t>(out)) & 15) == 0,
            "flash_attn_fwd: pointers must be 16-byte aligned");
   SMBV_ARG(scale > 0.f, "flash_attn_fwd: scale must be positive");
+  SMBV_ARG(variant == 0, "flash_attn_fwd: variant=%d is reserved and must be 0", variant);
   const int BH = B * H;
   CUtensorMap tq, tk, tv;
   int r;
   if ((r = attn_tmap(&tq, q, BH, N, ATT_BQ))) return r;
   if ((r = attn_tmap(&tk, k, BH, N, ATT_BK))) return r;
-  if (v_kmajor == 1) {
-    SMBV_ARG(N % 8 == 0, "flash_attn_fwd: V^T layout needs N %% 8 == 0");
-    uint64_t dims[3] = {(uint64_t)N, 64, (uint64_t)BH};
-    uint64_t str[2] = {(uint64_t)N * 2, (uint64_t)N * 64 * 2};
-    uint32_t box[3] = {64, 64, 1};
-    if ((r = make_tmap(&tv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, v, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B))) return r;
-  } else {
-    if ((r = attn_tmap(&tv, v, BH, N, ATT_BK))) return r;
-  }
+  if ((r = attn_tmap(&tv, v, BH, N, ATT_BK))) return r;
   static bool attr_set = false;
   if (!attr_set) {
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM));
+    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, A2_SMEM));
     attr_set = true;
   }
   const float scale_log2 = scale * 1.4426950408889634f;
   __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
-  if (v_kmajor == 0 || v_kmajor >= 10) {  // default kernel: two query tiles per CTA; 10..13 select the exp2-emulation share
-    // whole units in complete waves; the units of a partial last wave are split by key range (see the kernel)
-    const int t128 = (N + ATT_BQ - 1) / ATT_BQ, pph = t128 / 2, num_pairs = BH * pph, odd = BH * (t128 & 1);
-    const int nkv_total = (N + ATT_BK - 1) / ATT_BK;
-    const int W = num_sms();
-    int n_full = num_pairs, n_split = 0, parts = 2;
-    {
-      const int rest = num_pairs % W, k = attn_fwd_parts(num_pairs, nkv_total);
-      const int64_t need = (int64_t)rest * k * 2 * ATT_BQ * 68 * (int64_t)sizeof(float);
-      if (k >= 2 && workspace && workspace_bytes >= need) n_split = rest, n_full = num_pairs - rest, parts = k;
-    }
-    dim3 grid2(n_full + parts * n_split + odd);
-    const int pph_arg = pph > 0 ? pph : 1;
-    float* wsf = reinterpret_cast<float*>(workspace);
-#define SMBV_ATTN2(MASK)                                                                                              \
-  do {                                                                                                                \
-    static bool set_ = false;                                                                                         \
-    if (!set_) {                                                                                                      \
-      SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd2_kernel<MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize, A2_SMEM)); \
-      set_ = true;                                                                                                    \
-    }                                                                                                                 \
-    flash_attn_fwd2_kernel<MASK><<<grid2, A2_THREADS, A2_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse, n_full, n_split, parts, pph_arg, wsf, stagger_ns); \
-  } while (0)
-#ifdef SMBV_DEV_BUILD  // `make DEV=1`: exp2-emulation shares, the four-warpgroup kernel and the timeline trace (tools/run_attn.py, trace_attn_fwd.py)
-    static const int stagger_ns = [] { const char* e = getenv("SMBV_ATTN_FWD_STAGGER_NS"); return e ? atoi(e) : 0; }();
-    static const bool use_v4 = [] { const char* e = getenv("SMBV_ATTN_FWD_V4"); return e && e[0] == '1'; }();
-#define SMBV_ATTN4(MASK)                                                                                              \
-  do {                                                                                                                \
-    static bool set_ = false;                                                                                         \
-    if (!set_) {                                                                                                      \
-      SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd4_kernel<MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize, A4_SMEM)); \
-      set_ = true;                                                                                                    \
-    }                                                                                                                 \
-    flash_attn_fwd4_kernel<MASK><<<grid2, A4_THREADS, A4_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse, n_full, n_split, parts, pph_arg, wsf); \
-  } while (0)
-    static const bool use_fold = [] { const char* e = getenv("SMBV_ATTN_FOLD"); return e && e[0] == '1'; }();
-    if (v_kmajor == 0 && use_fold) {
-      static bool setf = false;
-      if (!setf) {
-        SMBV_CUDA(cudaFuncSetAttribute(flash_attn_fwd2_kernel<0xA4A4u, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, A2_SMEM));
-        setf = true;
-      }
-      flash_attn_fwd2_kernel<0xA4A4u, true><<<grid2, A2_THREADS, A2_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse, n_full, n_split, parts, pph_arg, wsf, 0);
-    } else
-    if (v_kmajor == 14 || (v_kmajor == 0 && use_v4)) SMBV_ATTN4(0x0000u);
-    else if (v_kmajor == 24) SMBV_ATTN4(0xA4A4u);
-    else if (v_kmajor == 25) SMBV_ATTN4(0xAAAAu);
-    else if (v_kmajor == 26) SMBV_ATTN4(0x2AAAu);
-    else
-    switch (v_kmajor) {
-      case 11: SMBV_ATTN2(0x8888u); break;  // 25 % of the exponentials on the FMA pipe
-      case 13: SMBV_ATTN2(0xAAAAu); break;  // 50 %
-      case 15: SMBV_ATTN2(0x1249u); break;  // 31.25 %
-      case 16: SMBV_ATTN2(0x2AAAu); break;  // 43.75 %
-      case 17: SMBV_ATTN2(0x9292u); break;  // 37.5 %, other placements of the six emulated pairs per 16
-      case 18: SMBV_ATTN2(0x4949u); break;
-      case 19: SMBV_ATTN2(0x00FCu); break;
-      case 10: SMBV_ATTN2(0x0000u); break;  // all MUFU.EX2
-      default: SMBV_ATTN2(0xA4A4u); break;
-    }
-#undef SMBV_ATTN4
-#else
-    // 6 of every 16 pairs (37.5 %) of the exponentials on the FMA / ALU pipes.  Measured on one box, same run: 1.52 ms vs
-    // 1.60 ms all-MUFU at H=12, N=20480 (-5 %; also -5 % at H=6 and at N=7168); 25 % and 31 % gain less, 44 % and 50 % fall off a
-    // cliff (1.78 / 1.85 ms: the softmax warps become issue-bound), other placements of the six pairs are 1-7 % slower.
-    constexpr int stagger_ns = 0;
-    SMBV_ARG(v_kmajor == 0, "flash_attn_fwd: unknown kernel selector %d (kernel variants need a `make DEV=1` build)", v_kmajor);
-    SMBV_ATTN2(0xA4A4u);
-#endif
-#undef SMBV_ATTN2
-    SMBV_LAUNCH_CHECK("flash_attn_fwd2");
-    if (n_split > 0) {
-      flash_attn_combine_kernel<<<(n_split * 2 * ATT_BQ + 7) / 8, 256, 0, (cudaStream_t)st>>>(wsf, n_full, n_split, parts, pph_arg, H, N, o, lse);
-      SMBV_LAUNCH_CHECK("flash_attn_combine");
-    }
-    return 0;
+  // whole units in complete waves; the units of a partial last wave are split by key range (see the kernel)
+  const int t128 = (N + ATT_BQ - 1) / ATT_BQ, pph = t128 / 2, num_pairs = BH * pph, odd = BH * (t128 & 1);
+  const int nkv_total = (N + ATT_BK - 1) / ATT_BK;
+  const int W = num_sms();
+  int n_full = num_pairs, n_split = 0, parts = 2;
+  {
+    const int rest = num_pairs % W, k = attn_fwd_parts(num_pairs, nkv_total);
+    const int64_t need = (int64_t)rest * k * 2 * ATT_BQ * 68 * (int64_t)sizeof(float);
+    if (k >= 2 && workspace && workspace_bytes >= need) n_split = rest, n_full = num_pairs - rest, parts = k;
   }
-  dim3 grid((N + ATT_BQ - 1) / ATT_BQ, BH);
-  if (v_kmajor == 1)
-    flash_attn_fwd_kernel<true><<<grid, ATT_THREADS, ATT_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse);
-  else
-    flash_attn_fwd_kernel<false><<<grid, ATT_THREADS, ATT_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse);
-  SMBV_LAUNCH_CHECK("flash_attn_fwd");
+  dim3 grid2(n_full + parts * n_split + odd);
+  const int pph_arg = pph > 0 ? pph : 1;
+  float* wsf = reinterpret_cast<float*>(workspace);
+  flash_attn_fwd2_kernel<<<grid2, A2_THREADS, A2_SMEM, (cudaStream_t)st>>>(tq, tk, tv, H, N, scale_log2, scale, o, lse, n_full,
+                                                                            n_split, parts, pph_arg, wsf);
+  SMBV_LAUNCH_CHECK("flash_attn_fwd2");
+  if (n_split > 0) {
+    flash_attn_combine_kernel<<<(n_split * 2 * ATT_BQ + 7) / 8, 256, 0, (cudaStream_t)st>>>(wsf, n_full, n_split, parts, pph_arg, H, N, o, lse);
+    SMBV_LAUNCH_CHECK("flash_attn_combine");
+  }
   return 0;
 }
 
@@ -1141,12 +421,3 @@ extern "C" int smbv_flash_attn_fwd(const smbv_bf16* q, const smbv_bf16* k, const
                                    float scale, smbv_bf16* out, float* lse, smbv_stream_t st) {
   return smbv_flash_attn_fwd_ex(q, k, v, B, H, N, scale, out, lse, 0, nullptr, 0, st);
 }
-
-#ifdef SMBV_DEV_BUILD
-// developer aid: copies the forward-kernel timeline trace (SMBV_ATTN_FWD_STAGGER_NS=-1) to the host; not in include/smbv_b200.h
-extern "C" int smbv_debug_read_fwd_trace(long long* dst) {
-  SMBV_CUDA(cudaDeviceSynchronize());
-  SMBV_CUDA(cudaMemcpyFromSymbol(dst, smbv::g_ftrace, sizeof(long long) * 12 * 32));
-  return 0;
-}
-#endif

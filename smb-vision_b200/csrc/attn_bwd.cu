@@ -21,19 +21,12 @@
 // Roles in both: warp 0 lane 0 TMA producer; warp 1 lane 0 issues the score products, warp 3 lane 0 the gradient
 // products; warp 2 stages lse/D (dkdv only); warpgroups 1,2 = 256 math threads, thread = TMEM lane, each warpgroup takes
 // 64 of the 128 score columns.  Scores of block n+1 and the gradient products of block n run under the math of block n+1.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "../../include/smbv_b200.h"
 
 namespace smbv {
 
-#ifndef SMBV_DQ_N128
-#define SMBV_DQ_N128 1
-#endif
-#ifndef SMBV_BWD_EMU_MASK
-#define SMBV_BWD_EMU_MASK 0xA4A4u  // pairs (of every 16) whose exponentials run on the FMA / ALU pipes instead of MUFU (0 = none)
-#endif
+constexpr uint32_t EX2_EMU_PAIRS = 0xA4A4u;  // pairs (of every 16) whose exponentials run on the FMA / ALU pipes instead of MUFU
 constexpr int AB_THREADS = 384;
 constexpr int AB_TILE = 128 * 64 * 2;  // 16 KB
 constexpr int AB_STAGES = 5;  // K/V (dQ kernel) or Q/dO (dK/dV kernel) prefetch depth: a 32 KB block takes ~1700 cycles from L2 under load
@@ -257,7 +250,7 @@ flash_attn_bwd_dkdv_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid
           // sv = S^T - lse/scale, dpv = dP^T - D (the statistics came in through the fifth K-step of the score products)
           const uint64_t x2 = fmul2(pack2(__uint_as_float(sv[col]), __uint_as_float(sv[col + 1])), sc2);
           float p0, p1;  // key rows past N (zero K/V rows) only feed accumulator rows that are never stored
-          if ((SMBV_BWD_EMU_MASK >> ((c * 8 + q) & 15)) & 1u) {
+          if ((EX2_EMU_PAIRS >> ((c * 8 + q) & 15)) & 1u) {
             ex2_emu2(x2, p0, p1);
           } else {
             float a0, a1;
@@ -318,17 +311,6 @@ flash_attn_bwd_dkdv_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid
 // ------------------------------------------------------------------------------------------------------------------
 // dQ kernel: CTA = 128 queries, streams key blocks
 // ------------------------------------------------------------------------------------------------------------------
-#ifdef SMBV_DEV_BUILD
-// timeline trace of CTA (0,0) for the first 24 key blocks (KNOCK == 7 only): g_trace[event][j] = clock64()
-__device__ long long g_trace[16][24];
-#define SMBV_TR(ev, j_)                                                                  \
-  do {                                                                                   \
-    if (KNOCK == 7 && blockIdx.x == 3 && blockIdx.y == 0 && (j_) < 24) g_trace[ev][j_] = clock64(); \
-  } while (0)
-#else
-#define SMBV_TR(ev, j_) do { } while (0)
-#endif
-template <int KNOCK>  // 0 = product kernel; 1..4 = timing-only knock-out variants (tools/run_attn_bwd.py, SMBV_DQ_KNOCK)
 __global__ void __launch_bounds__(AB_THREADS, 1)
 flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                          const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmDO, int H, int N,
@@ -398,14 +380,13 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
         tma_load_3d(smem_u32(sK + s * AB_TILE), &tmK, smem_u32(&k_full[s]), 0, j * 128, bh);
         mbar_expect_tx(smem_u32(&v_full[s]), AB_TILE);
         tma_load_3d(smem_u32(sV + s * AB_TILE), &tmV, smem_u32(&v_full[s]), 0, j * 128, bh);
-        SMBV_TR(0, j);
         if (++s == AB_STAGES) s = 0, ph ^= 1;
       }
     } else if (warp == 1 && elect_one()) {  // ===== MMA issuer A: S = Q K_j^T, dP = dO V_j^T for the whole 128-key block =====
       // A tcgen05.mma costs the issuing thread ~75 cycles regardless of its size (timeline trace, profiles/r01_attn_notes.md):
       // with 64-key halves (N = 64, 32 tensor-pipe cycles each) the 16 issues + 4 commits per block WERE the 1790-cycle block
       // period.  N = 128 halves the issue count; one commit serves both math warpgroups.
-      constexpr uint32_t id_s = umma_idesc(UMMA_BF16, 128, SMBV_DQ_N128 ? 128 : 64, 0, 0);
+      constexpr uint32_t id_s = umma_idesc(UMMA_BF16, 128, 128, 0, 0);
       const uint64_t dQ_k = umma_desc(smem_u32(sQ), 16, 1024, UMMA_SW_128B);
       const uint64_t dDO_k = umma_desc(smem_u32(sDO), 16, 1024, UMMA_SW_128B);
       const uint64_t dK_k = umma_desc(smem_u32(sK), 16, 1024, UMMA_SW_128B);
@@ -415,13 +396,9 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
       for (int j = 0; j < nkv; ++j) {
         mbar_wait(smem_u32(&k_full[s]), ph);
         mbar_wait(smem_u32(&v_full[s]), ph);
-        SMBV_TR(1, j);
-#if SMBV_DQ_N128
         if (j > 0) {  // both halves of block j-1 are in registers
           mbar_wait(smem_u32(&s_free[0]), (j - 1) & 1);
-          SMBV_TR(2, j);
           mbar_wait(smem_u32(&s_free[1]), (j - 1) & 1);
-          SMBV_TR(3, j);
         }
         tc_fence_after();
         const uint64_t off = (uint64_t)((s * AB_TILE) >> 4);
@@ -432,22 +409,6 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
         umma_commit(smem_u32(&s_full[0]));      // both math warpgroups wait on this one
         umma_commit(smem_u32(&k_empty[s]));     // (second arrival: issuer B; V_j is only read here, so k_empty covers it too)
         if (++s == AB_STAGES) s = 0, ph ^= 1;
-#else
-#pragma unroll
-        for (int w = 0; w < 2; ++w) {
-          if (j > 0) mbar_wait(smem_u32(&s_free[w]), (j - 1) & 1);
-          SMBV_TR(2 + w, j);
-          tc_fence_after();
-          const uint64_t off = (uint64_t)((s * AB_TILE + w * 8192) >> 4);  // key rows [64w, 64w+64) of the stage
-#pragma unroll
-          for (int k = 0; k < 4; ++k) umma_f16_ss(T_S + w * 64, dQ_k + 2 * k, dK_k + off + 2 * k, id_s, k != 0);
-#pragma unroll
-          for (int k = 0; k < 4; ++k) umma_f16_ss(T_DP + w * 64, dDO_k + 2 * k, dV_k + off + 2 * k, id_s, k != 0);
-          umma_commit(smem_u32(&s_full[w]));
-        }
-        umma_commit(smem_u32(&k_empty[s]));     // (second arrival: issuer B; V_j is only read here, so k_empty covers it too)
-        if (++s == AB_STAGES) s = 0, ph ^= 1;
-#endif
       }
     } else if (warp == 3 && elect_one()) {  // ===== MMA issuer B: dQ += dS K_j, per half =====
       constexpr uint32_t id_g = umma_idesc(UMMA_BF16, 128, 64, 0, 1);
@@ -458,12 +419,11 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
 #pragma unroll
         for (int w = 0; w < 2; ++w) {
           mbar_wait(smem_u32(&p_full[w]), j & 1);
-          SMBV_TR(4 + w, j);
           tc_fence_after();
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             const int kk = w * 4 + k;
-            if (KNOCK != 5) umma_f16_ts(T_DQ, T_DS + kk * 8, dK_mn + off + (uint64_t)(kk * 128), id_g, (j | kk) != 0);
+            umma_f16_ts(T_DQ, T_DS + kk * 8, dK_mn + off + (uint64_t)(kk * 128), id_g, (j | kk) != 0);
           }
           umma_commit(smem_u32(&pd_done[w]));
         }
@@ -489,27 +449,15 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
     const float dsum = q_ok ? Dsum[(int64_t)bh * n_local + qrow] : 0.f;
     const uint64_t sc2 = pack2(scale_log2, scale_log2), nl2_row = pack2(neg_l2, neg_l2), nds2 = pack2(-dsum, -dsum);
     for (int j = 0; j < nkv_m; ++j) {
-      mbar_wait(smem_u32(&s_full[SMBV_DQ_N128 ? 0 : wg]), j & 1);
-      if (quad == 0 && lane == 0) SMBV_TR(6 + wg, j);
+      mbar_wait(smem_u32(&s_full[0]), j & 1);
       tc_fence_after();
       uint32_t dd[32];
       uint32_t sv[64], dpv[64];
-      if (KNOCK != 6) {
-        tmem_ld32(T_S + lane_base + wg * 64, *reinterpret_cast<uint32_t(*)[32]>(&sv[0]));
-        tmem_ld32(T_S + lane_base + wg * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&sv[32]));
-      } else {
-#pragma unroll
-        for (int q = 0; q < 64; ++q) sv[q] = (uint32_t)(j + q);
-      }
-      if (KNOCK != 4 && KNOCK != 6) {
-        tmem_ld32(T_DP + lane_base + wg * 64, *reinterpret_cast<uint32_t(*)[32]>(&dpv[0]));
-        tmem_ld32(T_DP + lane_base + wg * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&dpv[32]));
-      } else {
-#pragma unroll
-        for (int q = 0; q < 64; ++q) dpv[q] = sv[q];
-      }
+      tmem_ld32(T_S + lane_base + wg * 64, *reinterpret_cast<uint32_t(*)[32]>(&sv[0]));
+      tmem_ld32(T_S + lane_base + wg * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&sv[32]));
+      tmem_ld32(T_DP + lane_base + wg * 64, *reinterpret_cast<uint32_t(*)[32]>(&dpv[0]));
+      tmem_ld32(T_DP + lane_base + wg * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&dpv[32]));
       tmem_wait_ld();
-      if (quad == 0 && lane == 0) SMBV_TR(8 + wg, j);
       tc_fence_before();
       __syncwarp();
       // the next block's scores run under this block's math — provided the arrive really precedes the math in the SASS:
@@ -526,9 +474,7 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
           const uint64_t x2 = ffma2(pack2(__uint_as_float(sv[col]), __uint_as_float(sv[col + 1])), sc2, nl2);
           float a0, a1, p0, p1;
           unpack2(x2, a0, a1);
-          if (KNOCK == 1 || KNOCK == 2 || KNOCK == 6) {
-            p0 = a0, p1 = a1;
-          } else if ((SMBV_BWD_EMU_MASK >> ((c * 8 + q) & 15)) & 1u) {
+          if ((EX2_EMU_PAIRS >> ((c * 8 + q) & 15)) & 1u) {
             ex2_emu2(x2, p0, p1);
           } else {
             p0 = ex2f(a0), p1 = ex2f(a1);
@@ -537,18 +483,15 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
           // multiplied by zero rows in dQ += dS K_j  (the per-element selects cost 134 of 327 instructions per block)
           float d0, d1;  // dS without the softmax scale: applied once to dQ in the epilogue
           unpack2(fmul2(pack2(p0, p1), fadd2(pack2(__uint_as_float(dpv[col]), __uint_as_float(dpv[col + 1])), nds2)), d0, d1);
-          dd[c * 8 + q] = KNOCK == 2 || KNOCK == 6 ? (sv[col] ^ dpv[col + 1]) : pack_bf16(d0, d1);
+          dd[c * 8 + q] = pack_bf16(d0, d1);
         }
       }
-      if (quad == 0 && lane == 0) SMBV_TR(10 + wg, j);
       if (j > 0) {
         mbar_wait(smem_u32(&pd_done[wg]), (j - 1) & 1);
         tc_fence_after();
       }
-      if (quad == 0 && lane == 0) SMBV_TR(12 + wg, j);
-      if (KNOCK != 3 || j == 0) tmem_st32(T_DS + lane_base + wg * 32, dd);
+      tmem_st32(T_DS + lane_base + wg * 32, dd);
       tmem_wait_st();
-      if (quad == 0 && lane == 0) SMBV_TR(14 + wg, j);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&p_full[wg]));
@@ -573,203 +516,6 @@ flash_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_c
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, 512);
 }
-
-#ifdef SMBV_DEV_BUILD  // experiment kept for the record (profiles/r01_attn_notes.md: parity-green, not faster); not in the release library
-// ------------------------------------------------------------------------------------------------------------------
-// dQ kernel, two query tiles per CTA ("dq2"): CTA = 256 queries (tiles A, B) of one head, streams 64-key blocks.
-//   per tile t:  S_t = Q_t K_j^T (SS, M128 N64)  dP_t = dO_t V_j^T  ->  dS_t bf16 -> TMEM  ->  dQ_t += dS_t K_j (TS)
-//   TMEM columns per tile: S 64 | dP 64 | dS 32 | dQ 64 = 224 (tile B at +256)
-// Each tile has its own MMA-issuing thread and its own math warpgroup (thread = query row, 64 key columns), like the forward
-// kernel: the TMEM load / store / barrier phases of one tile fall into the math (MUFU) phase of the other, which the
-// one-tile kernel could not do (timeline trace: 1370 cycles of math + 280 cycles of exposed load / store / wait per block),
-// and K / V are streamed once per 256 queries instead of once per 128.
-// ------------------------------------------------------------------------------------------------------------------
-constexpr int DQ2_STAGES = 6;
-constexpr int DQ2_KV_TILE = 64 * 64 * 2;  // 8 KB: 64 keys x 64 d
-constexpr int DQ2_SMEM = 4 * AB_TILE + 2 * DQ2_STAGES * DQ2_KV_TILE + 1024 + 256;
-
-__global__ void __launch_bounds__(AB_THREADS, 1)
-flash_attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK64,
-                          const __grid_constant__ CUtensorMap tmV64, const __grid_constant__ CUtensorMap tmDO, int H, int N,
-                          float scale, const float* __restrict__ lse, const float* __restrict__ Dsum,
-                          __nv_bfloat16* __restrict__ dq, int zero) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;                       // 2 tiles
-  uint8_t* sDO = sQ + 2 * AB_TILE;          // 2 tiles
-  uint8_t* sK = sDO + 2 * AB_TILE;          // DQ2_STAGES x 8 KB
-  uint8_t* sV = sK + DQ2_STAGES * DQ2_KV_TILE;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + DQ2_STAGES * DQ2_KV_TILE);
-  uint64_t* q_full = bars;                        // 1
-  uint64_t* kv_full = q_full + 1;                 // [STAGES]
-  uint64_t* kv_empty = kv_full + DQ2_STAGES;      // [STAGES] count ntiles (each tile's issuer, after its dQ product)
-  uint64_t* s_full = kv_empty + DQ2_STAGES;       // [2] per tile
-  uint64_t* s_free = s_full + 2;                  // [2] 4 warps
-  uint64_t* p_full = s_free + 2;                  // [2] 4 warps
-  uint64_t* pd_done = p_full + 2;                 // [2]
-  uint64_t* acc_full = pd_done + 2;               // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * 256;
-  const int bh = blockIdx.y;
-  const int ntiles = (q0 + 128 < N) ? 2 : 1;
-  const int nb = (N + 63) / 64;
-  const float scale_log2 = scale * 1.4426950408889634f;
-
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK64);
-    tma_prefetch_desc(&tmV64);
-    tma_prefetch_desc(&tmDO);
-    mbar_init(smem_u32(q_full), 1);
-    for (int s = 0; s < DQ2_STAGES; ++s) mbar_init(smem_u32(&kv_full[s]), 1), mbar_init(smem_u32(&kv_empty[s]), ntiles);
-    for (int t = 0; t < 2; ++t) {
-      mbar_init(smem_u32(&s_full[t]), 1);
-      mbar_init(smem_u32(&s_free[t]), 4);
-      mbar_init(smem_u32(&p_full[t]), 4);
-      mbar_init(smem_u32(&pd_done[t]), 1);
-      mbar_init(smem_u32(&acc_full[t]), 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) tmem_alloc(smem_u32(tmem_slot), 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < 4) {
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 72;");
-    if (warp == 0 && elect_one()) {  // ===== TMA producer =====
-      mbar_expect_tx(smem_u32(q_full), 2 * ntiles * AB_TILE);
-      for (int t = 0; t < ntiles; ++t) {
-        tma_load_3d(smem_u32(sQ + t * AB_TILE), &tmQ, smem_u32(q_full), 0, q0 + t * 128, bh);
-        tma_load_4d(smem_u32(sDO + t * AB_TILE), &tmDO, smem_u32(q_full), 0, q0 + t * 128, bh % H, bh / H);
-      }
-      uint32_t s = 0, ph = 0;
-      for (int j = 0; j < nb; ++j) {
-        mbar_wait(smem_u32(&kv_empty[s]), ph ^ 1);
-        mbar_expect_tx(smem_u32(&kv_full[s]), 2 * DQ2_KV_TILE);
-        tma_load_3d(smem_u32(sK + s * DQ2_KV_TILE), &tmK64, smem_u32(&kv_full[s]), 0, j * 64, bh);
-        tma_load_3d(smem_u32(sV + s * DQ2_KV_TILE), &tmV64, smem_u32(&kv_full[s]), 0, j * 64, bh);
-        if (++s == DQ2_STAGES) s = 0, ph ^= 1;
-      }
-    } else if ((warp == 1 || (warp == 2 && ntiles == 2)) && elect_one()) {  // ===== MMA issuers: warp 1 -> tile A, warp 2 -> tile B =====
-      const int t = warp - 1;
-      constexpr uint32_t id_s = umma_idesc(UMMA_BF16, 128, 64, 0, 0);
-      constexpr uint32_t id_g = umma_idesc(UMMA_BF16, 128, 64, 0, 1);  // A (dS) in TMEM, B = K_j read MN-major
-      const uint64_t dQ_k = umma_desc(smem_u32(sQ + t * AB_TILE), 16, 1024, UMMA_SW_128B);
-      const uint64_t dDO_k = umma_desc(smem_u32(sDO + t * AB_TILE), 16, 1024, UMMA_SW_128B);
-      const uint64_t dK_k = umma_desc(smem_u32(sK), 16, 1024, UMMA_SW_128B);
-      const uint64_t dV_k = umma_desc(smem_u32(sV), 16, 1024, UMMA_SW_128B);
-      const uint64_t dK_mn = umma_desc(smem_u32(sK), DQ2_KV_TILE, 1024, UMMA_SW_128B);
-      const uint32_t T_S = tmem_base + t * 256, T_DP = T_S + 64, T_DS = T_S + 128, T_DQ = T_S + 160;
-      uint32_t ss = 0, sph = 0, gs = 0;
-      auto issue_scores = [&]() {  // S_t, dP_t of the block in stage ss
-        mbar_wait(smem_u32(&kv_full[ss]), sph);
-        tc_fence_after();
-        const uint64_t off = (uint64_t)((ss * DQ2_KV_TILE) >> 4);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) umma_f16_ss(T_S, dQ_k + 2 * k, dK_k + off + 2 * k, id_s, k != 0);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) umma_f16_ss(T_DP, dDO_k + 2 * k, dV_k + off + 2 * k, id_s, k != 0);
-        umma_commit(smem_u32(&s_full[t]));
-        if (++ss == DQ2_STAGES) ss = 0, sph ^= 1;
-      };
-      mbar_wait(smem_u32(q_full), 0);
-      issue_scores();
-      for (int j = 0; j < nb; ++j) {
-        if (j + 1 < nb) {  // scores of block j+1 as soon as block j sits in registers: they run under the math of block j
-          mbar_wait(smem_u32(&s_free[t]), j & 1);
-          issue_scores();
-        }
-        mbar_wait(smem_u32(&p_full[t]), j & 1);
-        tc_fence_after();
-        const uint64_t off = (uint64_t)((gs * DQ2_KV_TILE) >> 4);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) umma_f16_ts(T_DQ, T_DS + k * 8, dK_mn + off + (uint64_t)(k * 128), id_g, (j | k) != 0);
-        umma_commit(smem_u32(&pd_done[t]));
-        umma_commit(smem_u32(&kv_empty[gs]));
-        if (++gs == DQ2_STAGES) gs = 0;
-      }
-      umma_commit(smem_u32(&acc_full[t]));
-    }
-    __syncwarp();
-  } else if ((warp >> 2) - 1 < ntiles) {  // ===== math: warpgroup = tile, thread = query row, 64 key columns per block =====
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 216;");
-    int n_local = N;
-    asm volatile("" : "+r"(n_local));
-    const int nb_m = (n_local + 63) / 64;
-    const int t = (warp >> 2) - 1;
-    const int quad = warp & 3;
-    const int r = quad * 32 + lane;
-    const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
-    const uint32_t T_S = tmem_base + lane_base + t * 256, T_DP = T_S + 64, T_DS = T_S + 128, T_DQ = T_S + 160;
-    const int qrow = q0 + t * 128 + r;
-    const bool q_ok = qrow < n_local;
-    // out-of-range query rows: lse = +inf -> P = 0
-    const float neg_l2 = q_ok ? -lse[(int64_t)bh * n_local + qrow] * 1.4426950408889634f : -INFINITY;
-    const float dsum = q_ok ? Dsum[(int64_t)bh * n_local + qrow] : 0.f;
-    const uint64_t sc2 = pack2(scale_log2, scale_log2), nl2_row = pack2(neg_l2, neg_l2), nds2 = pack2(-dsum, -dsum);
-    for (int j = 0; j < nb_m; ++j) {
-      mbar_wait(smem_u32(&s_full[t]), j & 1);
-      tc_fence_after();
-      uint32_t sv[64], dpv[64], dd[32];
-      tmem_ld32(T_S, *reinterpret_cast<uint32_t(*)[32]>(&sv[0]));
-      tmem_ld32(T_S + 32, *reinterpret_cast<uint32_t(*)[32]>(&sv[32]));
-      tmem_ld32(T_DP, *reinterpret_cast<uint32_t(*)[32]>(&dpv[0]));
-      tmem_ld32(T_DP + 32, *reinterpret_cast<uint32_t(*)[32]>(&dpv[32]));
-      tmem_wait_ld();
-      tc_fence_before();
-      __syncwarp();
-      uint32_t tok = 0;  // the token dependency keeps the arrive above the exponentials in the SASS (see the one-tile kernel)
-      if (lane == 0) tok = mbar_arrive_tok(smem_u32(&s_free[t]));
-      const float zf = __uint_as_float(tok & (uint32_t)zero);
-      const uint64_t nl2 = fadd2(nl2_row, pack2(zf, zf));
-#pragma unroll
-      for (int q = 0; q < 32; ++q) {
-        const int col = 2 * q;
-        float a0, a1;
-        unpack2(ffma2(pack2(__uint_as_float(sv[col]), __uint_as_float(sv[col + 1])), sc2, nl2), a0, a1);
-        const float p0 = ex2f(a0), p1 = ex2f(a1);  // key rows past N: zero K rows make their dS irrelevant in dQ += dS K
-        float d0, d1;
-        unpack2(fmul2(pack2(p0, p1), fadd2(pack2(__uint_as_float(dpv[col]), __uint_as_float(dpv[col + 1])), nds2)), d0, d1);
-        dd[q] = pack_bf16(d0, d1);
-      }
-      if (j > 0) {  // dQ product of block j-1 still reads dS
-        mbar_wait(smem_u32(&pd_done[t]), (j - 1) & 1);
-        tc_fence_after();
-      }
-      tmem_st32(T_DS, dd);
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&p_full[t]));
-    }
-    mbar_wait(smem_u32(&acc_full[t]), 0);
-    tc_fence_after();
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      uint32_t o[32];
-      tmem_ld32(T_DQ + c * 32, o);
-      tmem_wait_ld();
-      if (q_ok) {
-        uint4* dst = reinterpret_cast<uint4*>(dq + ((int64_t)bh * n_local + qrow) * 64 + c * 32);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          dst[q] = make_uint4(pack_bf16(__uint_as_float(o[8 * q]) * scale, __uint_as_float(o[8 * q + 1]) * scale),
-                              pack_bf16(__uint_as_float(o[8 * q + 2]) * scale, __uint_as_float(o[8 * q + 3]) * scale),
-                              pack_bf16(__uint_as_float(o[8 * q + 4]) * scale, __uint_as_float(o[8 * q + 5]) * scale),
-                              pack_bf16(__uint_as_float(o[8 * q + 6]) * scale, __uint_as_float(o[8 * q + 7]) * scale));
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_base, 512);
-}
-#endif  // SMBV_DEV_BUILD
 
 // ------------------------------------------------------------------------------------------------------------------
 // Fused backward ("one pass"): the dK/dV kernel above additionally forms dQ_i = dS_i K_j for every block pair, so S / dP / the
@@ -1078,7 +824,7 @@ flash_attn_bwd_fused_kernel(const __grid_constant__ CUtensorMap tmQ, const __gri
           // sv = S^T - lse/scale, dpv = dP^T - D (the statistics came in through the fifth K-step of the score products)
           const uint64_t x2 = fmul2(pack2(__uint_as_float(sv[col]), __uint_as_float(sv[col + 1])), sc2);
           float p0, p1;
-          if ((SMBV_BWD_EMU_MASK >> ((c * 8 + q) & 15)) & 1u) {
+          if ((EX2_EMU_PAIRS >> ((c * 8 + q) & 15)) & 1u) {
             ex2_emu2(x2, p0, p1);
           } else {
             float a0, a1;
@@ -1205,10 +951,10 @@ __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const __nv_bfloat16*
   }
 }
 
-static int head_tmap(CUtensorMap* m, const void* base, int BH, int N, uint32_t rows = 128) {  // head-major [BH, N, 64]
+static int head_tmap(CUtensorMap* m, const void* base, int BH, int N) {  // head-major [BH, N, 64]
   uint64_t dims[3] = {64, (uint64_t)N, (uint64_t)BH};
   uint64_t str[2] = {64 * 2, (uint64_t)N * 64 * 2};
-  uint32_t box[3] = {64, rows, 1};
+  uint32_t box[3] = {64, 128, 1};
   return make_tmap(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
@@ -1243,16 +989,7 @@ extern "C" int smbv_flash_attn_bwd_ex(const smbv_bf16* q, const smbv_bf16* k, co
   static bool attr_set = false;
   if (!attr_set) {
     SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dkdv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DK_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-#ifdef SMBV_DEV_BUILD
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
-#endif
+    SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AB_SMEM));
     attr_set = true;
   }
   dim3 grid((N + 127) / 128, BH);
@@ -1261,8 +998,7 @@ extern "C" int smbv_flash_attn_bwd_ex(const smbv_bf16* q, const smbv_bf16* k, co
   // start on the SMs the last dK/dV wave leaves idle: 13 waves instead of 7 + 7.  Fork/join is by events (no host sync).
   static thread_local cudaStream_t s2 = nullptr;
   static thread_local cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  static const bool overlap = [] { const char* e = getenv("SMBV_ATTN_BWD_OVERLAP"); return !(e && e[0] == '0'); }();
-  const bool fork = overlap && ((int64_t)grid.x * grid.y) % num_sms() != 0;
+  const bool fork = ((int64_t)grid.x * grid.y) % num_sms() != 0;
   if (fork && !s2) {
     SMBV_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
     SMBV_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
@@ -1274,46 +1010,13 @@ extern "C" int smbv_flash_attn_bwd_ex(const smbv_bf16* q, const smbv_bf16* k, co
     SMBV_CUDA(cudaStreamWaitEvent(s2, ev_fork, 0));
     sq = s2;
   }
-#ifdef SMBV_DEV_BUILD  // `make DEV=1` only: knock-out / trace variants (WRONG results by design) and the two-tile dQ experiment
-  static const bool dev_hooks = [] { const char* e = getenv("SMBV_DEV_HOOKS"); return e && e[0] == '1'; }();
-  static const bool skip_dkdv = dev_hooks && getenv("SMBV_SKIP_DKDV") != nullptr;
-  static const int knock = [] { const char* e = getenv("SMBV_DQ_KNOCK"); return e ? atoi(e) : 0; }() * (dev_hooks ? 1 : 0);
-  static const bool use_dq2 = [] { const char* e = getenv("SMBV_ATTN_BWD_DQ2"); return e && e[0] == '1'; }();
-#else
-  constexpr bool skip_dkdv = false;
-#endif
   if (ev_dkdv_start) SMBV_CUDA(cudaEventRecord((cudaEvent_t)ev_dkdv_start, s));
-  if (!skip_dkdv)
   flash_attn_bwd_dkdv_kernel<<<grid, AB_THREADS, DK_SMEM, s>>>(tq, tk, tv, tdo, H, N, scale, lse, dsum_ws,
                                                                reinterpret_cast<__nv_bfloat16*>(dk), reinterpret_cast<__nv_bfloat16*>(dv), 0);
   SMBV_LAUNCH_CHECK("flash_attn_bwd_dkdv");
   if (ev_dkdv_stop) SMBV_CUDA(cudaEventRecord((cudaEvent_t)ev_dkdv_stop, s));
-#define SMBV_DQ_LAUNCH(K_) flash_attn_bwd_dq_kernel<K_><<<grid, AB_THREADS, AB_SMEM, sq>>>(tq, tk, tv, tdo, H, N, scale, lse, dsum_ws, reinterpret_cast<__nv_bfloat16*>(dq), 0)
-#ifdef SMBV_DEV_BUILD
-  if (use_dq2 && knock == 0) {
-    CUtensorMap tk64, tv64;
-    if ((r = head_tmap(&tk64, k, BH, N, 64))) return r;
-    if ((r = head_tmap(&tv64, v, BH, N, 64))) return r;
-    static bool set2 = false;
-    if (!set2) {
-      SMBV_CUDA(cudaFuncSetAttribute(flash_attn_bwd_dq2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ2_SMEM));
-      set2 = true;
-    }
-    dim3 grid2(((N + 127) / 128 + 1) / 2, BH);
-    flash_attn_bwd_dq2_kernel<<<grid2, AB_THREADS, DQ2_SMEM, sq>>>(tq, tk64, tv64, tdo, H, N, scale, lse, dsum_ws,
-                                                                  reinterpret_cast<__nv_bfloat16*>(dq), 0);
-  } else
-  if (knock == 1) SMBV_DQ_LAUNCH(1);
-  else if (knock == 2) SMBV_DQ_LAUNCH(2);
-  else if (knock == 3) SMBV_DQ_LAUNCH(3);
-  else if (knock == 4) SMBV_DQ_LAUNCH(4);
-  else if (knock == 5) SMBV_DQ_LAUNCH(5);
-  else if (knock == 6) SMBV_DQ_LAUNCH(6);
-  else if (knock == 7) SMBV_DQ_LAUNCH(7);
-  else
-#endif
-  SMBV_DQ_LAUNCH(0);
-#undef SMBV_DQ_LAUNCH
+  flash_attn_bwd_dq_kernel<<<grid, AB_THREADS, AB_SMEM, sq>>>(tq, tk, tv, tdo, H, N, scale, lse, dsum_ws,
+                                                             reinterpret_cast<__nv_bfloat16*>(dq), 0);
   SMBV_LAUNCH_CHECK("flash_attn_bwd_dq");
   if (fork) {
     SMBV_CUDA(cudaEventRecord(ev_join, s2));
@@ -1412,12 +1115,3 @@ extern "C" int smbv_flash_attn_bwd(const smbv_bf16* q, const smbv_bf16* k, const
                                    float* dsum_ws, smbv_bf16* dq, smbv_bf16* dk, smbv_bf16* dv, smbv_stream_t st) {
   return smbv_flash_attn_bwd_ex(q, k, v, o, dout, lse, B, H, N, scale, dsum_ws, dq, dk, dv, nullptr, nullptr, st);
 }
-
-#ifdef SMBV_DEV_BUILD
-// developer aid: copies the dQ-kernel timeline trace (SMBV_DQ_KNOCK=7) to the host; not part of include/smbv_b200.h
-extern "C" int smbv_debug_read_dq_trace(long long* dst) {
-  SMBV_CUDA(cudaDeviceSynchronize());
-  SMBV_CUDA(cudaMemcpyFromSymbol(dst, smbv::g_trace, sizeof(long long) * 16 * 24));
-  return 0;
-}
-#endif

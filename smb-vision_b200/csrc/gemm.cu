@@ -9,8 +9,6 @@
 //                                  (modes with a per-element side input: warps 2..5, registers -> global)
 #include <cstring>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "../../include/smbv_b200.h"
 
@@ -38,7 +36,6 @@ struct GemmCfg {
 struct GemmEpi {
   int M, N, K;
   int split_k;           // > 1: the K range is split over blockIdx-derived slices, epilogue must be a reducing one
-  int n_whole;           // output tiles [0, n_whole) run their whole K range, only the rest is cut into split_k slices (0: all are cut)
   const void* aux;       // EPI_DGELU_BF16: pre-activation, bf16 [M, ldo]
   const float* alpha;    // optional device scalar multiplied into the accumulator (EPI_ATOMIC_F32 / EPI_BF16 / EPI_F32)
   const float* bias;
@@ -263,18 +260,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int total_kb = (e.K + GEMM_BK - 1) / GEMM_BK;
   const int kb_per = (total_kb + e.split_k - 1) / e.split_k;
-  // work-unit id t: t < n_whole = output tile t with its whole K range; above = (output tile, K slice), slice fastest.  The reducing
-  // epilogues (fp32 TMA reduce-add: residual update, weight gradients) make a K split free of any workspace, so the output tiles of a
-  // PARTIAL LAST ROUND are cut into slices (480 tiles on 148 SMs: 3 rounds + 36 tiles x 4 slices = 3.25 rounds instead of 4)
-  const int n_whole = e.n_whole;
-  const int num_tiles = n_whole + (tiles_m * tiles_n - n_whole) * e.split_k;
+  // work-unit id t = (output tile, K slice), slice fastest.  split_k > 1 only with the fp32 reducing epilogue (weight gradients):
+  // the slices of one tile add their partial sums into the output, so a K split needs no workspace
+  const int num_tiles = tiles_m * tiles_n * e.split_k;
   auto decode = [&](int t, int& mn, int& slice, int& kb0, int& kb1) {
-    if (t < n_whole) {
-      mn = t, slice = 0, kb0 = 0, kb1 = total_kb;
-    } else {
-      const int u = t - n_whole, q = u / e.split_k;
-      mn = n_whole + q, slice = u - q * e.split_k, kb0 = slice * kb_per, kb1 = min(total_kb, kb0 + kb_per);
-    }
+    mn = t / e.split_k, slice = t - mn * e.split_k, kb0 = slice * kb_per, kb1 = min(total_kb, kb0 + kb_per);
   };
 
   if (threadIdx.x == 0) {
@@ -678,7 +668,7 @@ static int launch_gemm(const GemmHost& h, cudaStream_t st) {
     SMBV_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<BN, A_MN, B_MN, A3D, TMA_EPI, EPI4>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     attr_set = true;
   }
-  const int grid = min(e.n_whole + (tiles_m * tiles_n - e.n_whole) * e.split_k, num_sms());
+  const int grid = min(tiles_m * tiles_n * e.split_k, num_sms());
   gemm_bf16_kernel<BN, A_MN, B_MN, A3D, TMA_EPI, EPI4><<<grid, TMA_EPI ? GEMM_THREADS_TMA : GEMM_THREADS_REG, Cfg::SMEM_BYTES, st>>>(tmA, tmB, tmC, tmAux, e, tiles_m, tiles_n);
   SMBV_LAUNCH_CHECK("gemm_bf16");
   return 0;
@@ -691,49 +681,23 @@ static int dispatch_gemm(GemmHost& h, cudaStream_t st) {
   const bool b_mn = h.w_layout == 1;
   const int total_kb = (e.K + GEMM_BK - 1) / GEMM_BK;
   // fewer than two waves of 128x256 tiles: BN=128 gives more tiles (better SM fill); otherwise BN=256 halves the A re-reads
-  // (measured with tools/gemm_bn_sweep.py after the elect.sync issue fix: 7168x768 outputs 477/849 vs 439/812 TF/s)
+  // (measured after the elect.sync issue fix: 7168x768 outputs 477/849 vs 439/812 TF/s)
   const int64_t tiles256 = (int64_t)((e.M + 127) / 128) * ((e.N + 255) / 256);
   const bool bn256 = (e.N % 256 == 0) && tiles256 * (e.split_k > 0 ? e.split_k : 1) >= 2 * num_sms();
-  int bn = bn256 ? 256 : 128;
-  {  // developer override for A/B timing (tools/gemm_bn_sweep.py): SMBV_GEMM_BN=128|256
-    static const int forced = [] { const char* v = getenv("SMBV_GEMM_BN"); return v ? atoi(v) : 0; }();
-    if (forced == 128 || (forced == 256 && e.N % 256 == 0)) bn = forced;
-  }
+  const int bn = bn256 ? 256 : 128;
   if (e.split_k == 0) {  // auto: fill the machine when the output has few tiles (weight gradients)
     const int64_t tiles = (int64_t)((e.M + 127) / 128) * ((e.N + bn - 1) / bn);
     int sk = 1;
     if (e.mode == SMBV_EPI_ATOMIC_F32 && tiles < num_sms()) { int64_t want = (2 * (int64_t)num_sms() + tiles - 1) / tiles; sk = (int)(want < total_kb ? want : total_kb); }
     e.split_k = sk < 1 ? 1 : sk;
   }
-  if (e.mode == SMBV_EPI_RESID_F32 && e.residual == e.out && e.split_k <= 1) {
-    // in-place residual update = fp32 TMA reduce-add: the tiles of a partial last round are cut into K slices (see the kernel).
-    // tail cost in units of one whole tile: rounds(k) * (1/k + fixed / total_kb), fixed ~ 3 k-blocks of epilogue + pipeline fill
-    // OPT-IN (SMBV_GEMM_TAIL_SPLIT=1): the slices of one tile reduce into X in arbitrary order, so the residual stream — and with it
-    // the embeddings — would no longer be bit-reproducible run to run; measured gain 8-15 % on the fc2 GEMMs = 0.5 % of a step.
-    static const bool on = [] { const char* v = getenv("SMBV_GEMM_TAIL_SPLIT"); return v && v[0] == '1'; }();
-    const int W = num_sms();
-    const int64_t tiles = (int64_t)((e.M + 127) / 128) * ((e.N + bn - 1) / bn);
-    const int R = (int)(tiles % W);
-    if (on && tiles > W && R > 0) {
-      const double fixed = 3.0 / total_kb;
-      double best_cost = 1.0 + fixed;
-      int best = 1;
-      for (int k = 2; k <= 8 && k <= total_kb; ++k) {
-        if ((int64_t)((total_kb + k - 1) / k) * (k - 1) >= total_kb) continue;  // would leave an empty slice
-        const double cost = (double)(((int64_t)R * k + W - 1) / W) * (1.0 / k + fixed);
-        if (cost < best_cost * 0.97) best_cost = cost, best = k;
-      }
-      if (best > 1) e.split_k = best, e.n_whole = (int)(tiles - R);
-    }
-  }
   while (e.split_k > 1 && (int64_t)((total_kb + e.split_k - 1) / e.split_k) * (e.split_k - 1) >= total_kb) --e.split_k;  // no empty slice
   const bool tma_epi = use_tma_epilogue(e);
   // the two-transfer epilogues (dGELU: pre-activation slab in, gradient slab out; GELU with the saved pre-activation: two slabs out)
   // run on the four-slab-buffer variant (plain row-major A; W [N,K] for the forward fc1, W [K,N] for the fc2 dgrad)
-  static const bool epi4_on = [] { const char* v = getenv("SMBV_GEMM_EPI4"); return !(v && v[0] == '0'); }();
   // (measured, tools/gemm_small_sweep.py: dGELU 51.9 -> 47.6 us at M=7168, K=768 and 68.4 -> 57.8 us at M=20480, K=384; GELU + pre 51.5 -> 49.3 us
   //  at K=384 but 43.6 -> 45.3 us at K=768, where the third stage is missed: only short main loops take it)
-  if (epi4_on && tma_epi && !a_mn && !a3d && e.aux && (e.mode == SMBV_EPI_DGELU_BF16 || (e.mode == SMBV_EPI_GELU_BF16 && e.K <= 512))) {
+  if (tma_epi && !a_mn && !a3d && e.aux && (e.mode == SMBV_EPI_DGELU_BF16 || (e.mode == SMBV_EPI_GELU_BF16 && e.K <= 512))) {
     if (bn == 256) return b_mn ? launch_gemm<256, false, true, false, true, true>(h, st) : launch_gemm<256, false, false, false, true, true>(h, st);
     return b_mn ? launch_gemm<128, false, true, false, true, true>(h, st) : launch_gemm<128, false, false, false, true, true>(h, st);
   }
@@ -785,7 +749,7 @@ extern "C" int smbv_gemm_bf16(const smbv_gemm_args* a, smbv_stream_t st) {
     SMBV_ARG(a->pos && a->row_map && a->ldpos >= a->N && a->ldpos % 4 == 0, "gemm_bf16: pos-gather epilogue needs pos,row_map,ldpos");
   GemmHost h{};
   h.A = a->A, h.lda = a->lda, h.a_layout = SMBV_A_ROWMAJOR, h.W = a->W, h.ldw = a->ldw, h.w_layout = 0;
-  h.e = GemmEpi{a->M, a->N, a->K, 1, 0, nullptr, nullptr, a->bias, a->epilogue, a->out, a->ldo, a->residual, a->heads, a->tokens, a->pos, a->ldpos, a->row_map};
+  h.e = GemmEpi{a->M, a->N, a->K, 1, nullptr, nullptr, a->bias, a->epilogue, a->out, a->ldo, a->residual, a->heads, a->tokens, a->pos, a->ldpos, a->row_map};
   return dispatch_gemm(h, (cudaStream_t)st);
 }
 
@@ -810,6 +774,6 @@ extern "C" int smbv_gemm_ex(const smbv_gemm_ex_args* a, smbv_stream_t st) {
   GemmHost h{};
   h.A = a->A, h.lda = a->lda, h.a_layout = a->a_layout, h.W = a->W, h.ldw = a->ldw, h.w_layout = a->w_layout;
   h.a_part_stride = a->a_part_stride;
-  h.e = GemmEpi{a->M, a->N, a->K, a->split_k, 0, a->aux, a->alpha, a->bias, a->epilogue, a->out, a->ldo, a->residual, a->heads, 0, nullptr, 0, nullptr};
+  h.e = GemmEpi{a->M, a->N, a->K, a->split_k, a->aux, a->alpha, a->bias, a->epilogue, a->out, a->ldo, a->residual, a->heads, 0, nullptr, 0, nullptr};
   return dispatch_gemm(h, (cudaStream_t)st);
 }

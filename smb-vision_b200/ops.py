@@ -171,8 +171,8 @@ def gemm(a, w, bias=None, epilogue=EPI_BF16, out=None, residual=None, heads=0, t
     return out
 
 
-def flash_attn_fwd(q, k, v, scale: float, return_lse: bool = False, v_kmajor: bool = False):
-    """q,k bf16 [B,H,N,64]; v bf16 [B,H,N,64] (or V^T [B,H,64,N] when v_kmajor) -> out bf16 [B,N,H*64]."""
+def flash_attn_fwd(q, k, v, scale: float, return_lse: bool = False):
+    """q,k,v bf16 [B,H,N,64] -> out bf16 [B,N,H*64]."""
     _chk(q, torch.bfloat16, "q")
     _chk(k, torch.bfloat16, "k")
     _chk(v, torch.bfloat16, "v")
@@ -181,10 +181,10 @@ def flash_attn_fwd(q, k, v, scale: float, return_lse: bool = False, v_kmajor: bo
         raise SmbvError(f"flash_attn_fwd: head_dim {D} not supported (64 only)")
     out = torch.empty((B, N, H * 64), dtype=torch.bfloat16, device=q.device)
     lse = torch.empty((B, H, N), dtype=torch.float32, device=q.device) if return_lse else None
-    wsb = 0 if v_kmajor else int(_lib.load().smbv_flash_attn_fwd_workspace_bytes(B, H, N))
+    wsb = int(_lib.load().smbv_flash_attn_fwd_workspace_bytes(B, H, N))
     ws = torch.empty((wsb,), dtype=torch.uint8, device=q.device) if wsb else None
     call("smbv_flash_attn_fwd_ex", _ptr(q), _ptr(k), _ptr(v), B, H, N, float(scale), _ptr(out), _ptr(lse),
-         1 if v_kmajor else 0, _ptr(ws), wsb, _stream())
+         0, _ptr(ws), wsb, _stream())
     return (out, lse) if return_lse else out
 
 

@@ -58,8 +58,10 @@ def test_argument_errors_are_reported_before_launch(lib):
     g.A = g.W = g.out = 16
     g.M, g.N, g.K, g.lda, g.ldw, g.ldo = 128, 100, 64, 64, 64, 100
     assert lib.smbv_gemm_bf16(ctypes.byref(g), None) < 0 and b"multiple of 32" in lib.smbv_last_error()
-    # V-JEPA entry points (SURVEY.md §8f rank 4)
     P16 = ctypes.c_void_p(16)
+    assert lib.smbv_flash_attn_fwd_ex(P16, P16, P16, 1, 1, 128, 0.125, P16, None, 1, None, 0, None) < 0
+    assert b"variant" in lib.smbv_last_error()
+    # V-JEPA entry points (SURVEY.md §8f rank 4)
     assert lib.smbv_rope3d(P16, None, 2, 1, 2, 8, 60, 4, 4, 0, None) < 0 and b"multiple of 8" in lib.smbv_last_error()
     assert lib.smbv_rope3d(None, None, 2, 1, 2, 8, 64, 4, 4, 0, None) < 0 and b"null" in lib.smbv_last_error()
     assert lib.smbv_rope3d(P16, None, 2, 1, 2, 8, 64, 4, 100000, 0, None) < 0 and b"max_pos" in lib.smbv_last_error()

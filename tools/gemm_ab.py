@@ -1,5 +1,5 @@
 """Forward GEMMs with their fused epilogues at the model shapes: parity vs fp32 torch + CUDA-event timings next to torch.matmul
-(cuBLAS, no epilogue).  SMBV_GEMM_TAIL_SPLIT=1 enables the (non-deterministic, opt-in) K split of the last round of the residual-epilogue GEMMs for an A/B.
+(cuBLAS, no epilogue).
 usage: python tools/gemm_ab.py [tag]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -1,5 +1,5 @@
 """Encoder-side (7168-token) and decoder-side GEMM shapes of the MIM training step vs torch.matmul (cuBLAS, no epilogue), forward / dgrad / wgrad.
-usage: python tools/gemm_small_sweep.py [tag]   (SMBV_GEMM_BN=128|256 forces the N tile)"""
+usage: python tools/gemm_small_sweep.py [tag]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

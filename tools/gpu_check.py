@@ -206,7 +206,7 @@ def g_gemm():
             torch_tflops=2 * M * N * K / ms_t / 1e9)
 
 
-def _attn_case(B, H, N, vk, scale=0.125, seed=0):
+def _attn_case(B, H, N, scale=0.125, seed=0):
     import torch
     from smb_vision_b200 import ops
     dev = "cuda"
@@ -214,8 +214,7 @@ def _attn_case(B, H, N, vk, scale=0.125, seed=0):
     q = torch.randn(B, H, N, 64, device=dev).to(torch.bfloat16)
     k = torch.randn(B, H, N, 64, device=dev).to(torch.bfloat16)
     v = torch.randn(B, H, N, 64, device=dev).to(torch.bfloat16)
-    vin = v.transpose(2, 3).contiguous() if vk else v
-    out, lse = ops.flash_attn_fwd(q, k, vin, scale, return_lse=True, v_kmajor=vk)
+    out, lse = ops.flash_attn_fwd(q, k, v, scale, return_lse=True)
     s = (q.float() @ k.float().transpose(-1, -2)) * scale
     ref = (torch.softmax(s, -1) @ v.float()).transpose(1, 2).reshape(B, N, H * 64)
     lref = torch.logsumexp(s, -1)
@@ -223,13 +222,12 @@ def _attn_case(B, H, N, vk, scale=0.125, seed=0):
     extra = {}
     if not fr < 1e-2:
         extra = dict(got=out[0, :2, :4].tolist(), want=ref[0, :2, :4].tolist())
-    rec(f"attn_B{B}H{H}N{N}_{'vT' if vk else 'v'}", fr < 1e-2, frob=fr, maxabs=mx, lse_err=(lse - lref).abs().max().item(), **extra)
+    rec(f"attn_B{B}H{H}N{N}", fr < 1e-2, frob=fr, maxabs=mx, lse_err=(lse - lref).abs().max().item(), **extra)
 
 
 def g_attn():
-    for vk in (False, True):
-        for B, H, N in [(1, 1, 128), (1, 2, 256), (2, 3, 1024), (1, 2, 216), (1, 1, 72), (1, 1, 384), (1, 2, 3000 if not vk else 3008)]:
-            _attn_case(B, H, N, vk)
+    for B, H, N in [(1, 1, 128), (1, 2, 256), (2, 3, 1024), (1, 2, 216), (1, 1, 72), (1, 1, 384), (1, 2, 3000)]:
+        _attn_case(B, H, N)
 
 
 def g_attn_big():
@@ -255,24 +253,9 @@ def g_attn_big():
         ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2).reshape(1, N, H * 64)
         fr, mx = relerr(out.float(), ref.float())
         ms = timeit(lambda: ops.flash_attn_fwd(q, k, v, 0.125), iters=5, warmup=2)
-        from smb_vision_b200 import _lib
-        import ctypes as C
-        o1 = torch.empty_like(out)
-        def vx(variant):
-            _lib.call("smbv_flash_attn_fwd_ex", C.c_void_p(q.data_ptr()), C.c_void_p(k.data_ptr()), C.c_void_p(v.data_ptr()), 1, H, N, 0.125,
-                      C.c_void_p(o1.data_ptr()), None, variant, None, 0, C.c_void_p(torch.cuda.current_stream().cuda_stream))
-        ms_v1 = timeit(lambda: vx(2), iters=5, warmup=2)
-        emu = {}
-        for var in (10, 11, 12, 13):  # exp2-emulation shares: only in a `make DEV=1` library
-            try:
-                vx(var)
-            except Exception:
-                break
-            fre, _ = relerr(o1.float(), ref.float())
-            emu[f"emu{var}"] = [round(timeit(lambda: vx(var), iters=5, warmup=2), 4), round(fre, 6)]
         ms_t = timeit(lambda: torch.nn.functional.scaled_dot_product_attention(q, k, v), iters=5, warmup=2)
         fl = 4.0 * N * N * 64 * H
-        rec(f"attn_time_H{H}N{N}", fr < 1e-2, frob_vs_sdpa=fr, ms=ms, tflops=fl / ms / 1e9, v1_ms=ms_v1, emu=emu,  torch_sdpa_ms=ms_t,
+        rec(f"attn_time_H{H}N{N}", fr < 1e-2, frob_vs_sdpa=fr, ms=ms, tflops=fl / ms / 1e9, torch_sdpa_ms=ms_t,
             torch_sdpa_tflops=fl / ms_t / 1e9)
 
 
