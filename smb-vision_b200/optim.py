@@ -6,8 +6,10 @@
 * ``smbv_sumsq_f32``  : squared global gradient norm into a device scalar (deterministic, no host sync);
 * ``smbv_adamw_step`` : clip scale + AdamW + refresh of the bf16 operand copy of every weight, one pass, 30 B / parameter.
 
-Weight decay is applied to the same parameter set ``Trainer.get_decay_parameter_names`` selects (everything except
-LayerNorm weights and names containing "bias").
+Weight decay is applied to the same parameter set ``Trainer.get_decay_parameter_names`` selects: everything except the
+parameters of ``nn.LayerNorm`` modules and names matching "bias", "layernorm", "rmsnorm", "norm" as a whole name
+component or "_norm" at the end of one (``training.ArenaLayout.decay_segments``).  So V-JEPA's ``norm1`` / ``norm2``
+LayerNorm weights are not decayed.
 """
 from __future__ import annotations
 
@@ -53,6 +55,9 @@ class FusedAdamW:
         # frozen parameters (requires_grad=False at construction, e.g. a frozen encoder under a fine-tuned head) are skipped
         frozen = [k for k, p in self.params.model.named_parameters() if not p.requires_grad]
         starts, flags = self.layout.decay_segments(frozen)
+        # the native backward writes a gradient for every parameter; torch's clip_grad_norm_ never sees a frozen one (its
+        # .grad is None), so those views are zeroed before the global norm
+        self._frozen_views = [self.layout.offsets[k] for k in frozen]  # (offset, count)
         self.seg_start = torch.tensor(starts, dtype=torch.int32, device=dev)
         self.seg_nodecay = torch.tensor(flags, dtype=torch.uint8, device=dev)
         self.norm_sq = torch.zeros(1, dtype=torch.float32, device=dev)
@@ -80,6 +85,8 @@ class FusedAdamW:
         st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
         clip = self.max_grad_norm is not None and self.max_grad_norm > 0
         if clip:
+            for o, n in self._frozen_views:
+                g[o:o + n].zero_()
             call("smbv_sumsq_f32", ops._ptr(g), g.numel(), ops._ptr(self.ws), ops._ptr(self.norm_sq), st)
         lr = self.current_lr()
         self.steps += 1

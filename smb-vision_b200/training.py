@@ -8,6 +8,7 @@ of backward is still running.
 """
 from __future__ import annotations
 
+import re
 from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
@@ -108,6 +109,9 @@ class SideQueue:
 # ----------------------------------------------------------------------------------------------
 ALIGN = 64  # elements: 256 B in the fp32 arenas, 128 B in the bf16 one (TMA operand bases need 16 B)
 PAD_SUFFIX = "k_bias_pad"  # pseudo entry between q_bias and v_bias: the constant zero k bias of reference :261
+# transformers Trainer.get_decay_parameter_names: no weight decay for parameters of nn.LayerNorm modules or for names (lower
+# case) matching one of these
+NO_DECAY_PATTERNS = re.compile(r"bias|layernorm|rmsnorm|(?:^|\.)norm(?:$|\.)|_norm(?:$|\.)")
 
 
 class ArenaLayout:
@@ -117,6 +121,8 @@ class ArenaLayout:
 
     def __init__(self, model):
         self.shapes: Dict[str, torch.Size] = {k: p.shape for k, p in model.named_parameters()}
+        self.layernorm_params = {f"{mn}.{pn}" if mn else pn for mn, m in model.named_modules() if isinstance(m, torch.nn.LayerNorm)
+                                 for pn, _ in m.named_parameters()}
         groups = order_groups(model)
         real = [n for g in groups for n in g if not n.endswith(PAD_SUFFIX)]
         assert set(real) == set(self.shapes) and len(real) == len(self.shapes), set(real) ^ set(self.shapes)
@@ -144,13 +150,15 @@ class ArenaLayout:
         return {k: flat[o:o + n].view(self.shapes[k]) for k, (o, n) in self.offsets.items() if k in self.shapes}
 
     def decay_segments(self, frozen=()):
-        """(start4 int32[], flag uint8[]) for smbv_adamw_step: flag 1 = weight decay off (LayerNorm weights and everything
-        whose name contains "bias": transformers Trainer.get_decay_parameter_names), flag 2 = frozen (`frozen`: names with
-        requires_grad=False — neither updated nor decayed, as torch.optim skips them); adjacent equal flags merged."""
+        """(start4 int32[], flag uint8[]) for smbv_adamw_step: flag 1 = weight decay off, with the rule of transformers
+        Trainer.get_decay_parameter_names (every parameter of an nn.LayerNorm module, and every name matching
+        NO_DECAY_PATTERNS, e.g. "bias", "layernorm", ".norm.", "_norm."; the k_bias_pad entries count as biases), flag 2 =
+        frozen (`frozen`: names with requires_grad=False — neither updated nor decayed, as torch.optim skips them); adjacent
+        equal flags merged."""
         starts, flags = [], []
         frozen = set(frozen)
         for name in self.order:
-            nd = 1 if ("bias" in name or "layernorm" in name or "norm." in name) else 0
+            nd = 1 if (name in self.layernorm_params or NO_DECAY_PATTERNS.search(name.lower())) else 0
             if name in frozen:
                 nd = 2
             if not flags or flags[-1] != nd:

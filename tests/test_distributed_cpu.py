@@ -125,6 +125,56 @@ def test_grad_arena_layout():
     assert lc.order[0] == "classifier.weight" and lc.offsets["classifier.weight"] == (0, 3 * 130)
 
 
+def _decay_models():
+    import transformers
+    from transformers import VJEPA2Config
+
+    from smb_vision_b200.modeling import B200VideoMAEForPreTraining, B200VideoMAEForVideoClassification
+    from smb_vision_b200.vjepa import B200VJEPA2Model
+
+    def cls(mean_pooling):
+        hc = ge.hf_config(ge.SMALL64)
+        hc.num_labels, hc.additional_features_size, hc.use_mean_pooling = 3, 2, mean_pooling
+        return B200VideoMAEForVideoClassification(hc)
+
+    vc = VJEPA2Config(patch_size=16, crop_size=64, frames_per_clip=64, tubelet_size=16, in_chans=1, hidden_size=128, num_attention_heads=2,
+                      num_hidden_layers=2, pred_hidden_size=64, pred_num_attention_heads=2, pred_num_hidden_layers=2, pred_num_mask_tokens=2)
+    return {"videomae-pretraining": lambda: B200VideoMAEForPreTraining(ge.hf_config(ge.SMALL64)),
+            "classification-mean-pooling": lambda: cls(True), "classification-cls-token": lambda: cls(False),
+            "vjepa": lambda: B200VJEPA2Model(vc), "upstream-vjepa": lambda: transformers.VJEPA2Model(vc),
+            "upstream-videomae-pretraining": lambda: transformers.VideoMAEForPreTraining(ge.hf_config(ge.SMALL64))}
+
+
+@pytest.mark.parametrize("kind", list(_decay_models()))
+def test_decay_segments_match_trainer(kind):
+    """FusedAdamW's weight-decay set is transformers Trainer's: flag 0 exactly for the names
+    Trainer.get_decay_parameter_names returns (which excludes every nn.LayerNorm parameter, so V-JEPA's norm1 / norm2
+    weights too), flag 1 for the rest and for the k_bias_pad entries."""
+    from transformers import Trainer
+
+    from smb_vision_b200.training import PAD_SUFFIX, ArenaLayout
+
+    model = _decay_models()[kind]()
+    lay = ArenaLayout(model)
+    starts, flags = lay.decay_segments()
+    assert starts[0] == 0 and starts == sorted(starts) and all(a != b for a, b in zip(flags, flags[1:]))
+    decay = set(Trainer.get_decay_parameter_names(None, model))
+    assert decay and decay <= set(lay.shapes)
+
+    def flag(name):
+        o = lay.offsets[name][0] // 4
+        return flags[max(i for i, s0 in enumerate(starts) if s0 <= o)]
+
+    got = {n: flag(n) for n in lay.order}
+    assert all(got[n] == 1 for n in lay.order if n.endswith(PAD_SUFFIX))
+    wrong = sorted(n for n in lay.shapes if got[n] != (0 if n in decay else 1))
+    assert not wrong, wrong
+    frozen = sorted(lay.shapes)[::3]
+    starts_f, flags_f = lay.decay_segments(frozen)
+    o = lay.offsets[frozen[0]][0] // 4
+    assert flags_f[max(i for i, s0 in enumerate(starts_f) if s0 <= o)] == 2
+
+
 def test_cosine_schedule_matches_transformers():
     from transformers import get_cosine_schedule_with_warmup
 

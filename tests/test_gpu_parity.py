@@ -1183,6 +1183,46 @@ def test_fused_adamw_leaves_frozen_parameters_alone(ops):
             assert not torch.equal(p.detach(), before[k]), k
 
 
+def test_fused_adamw_clip_norm_ignores_frozen_parameters(ops):
+    """With a frozen patch embedding and decoder head, the global norm FusedAdamW clips by is clip_grad_norm_ over the
+    trainable parameters' gradients (a frozen parameter has no .grad under torch), although the native backward writes a
+    gradient for every parameter.  Control: the norm over the whole gradient arena, frozen gradients included (what the
+    optimiser computed before it zeroed them), is off by far more than the bound."""
+    from smb_vision_b200.modeling import B200VideoMAEForPreTraining, _prep_mask
+    from smb_vision_b200.optim import FusedAdamW
+    from smb_vision_b200.training import DataParallelStep
+
+    cfg = vo.OracleConfig(**ge.SMALL64)
+    model = B200VideoMAEForPreTraining(ge.hf_config(ge.SMALL64)).to(DEV)
+    model.load_state_dict(vo.synthetic_state_dict(cfg, 1234), strict=True)
+    # the patch embedding's gradient is small in this model, the decoder head's is not: freeze both
+    frozen = ["videomae.embeddings.patch_embeddings.projection.weight", "decoder.head.weight"]
+    for k in frozen:
+        model.get_parameter(k).requires_grad = False
+    opt = FusedAdamW(model, lr=1e-3)
+    dp = DataParallelStep(model, optimizer=opt)
+    x = vo.synthetic_volume(cfg, 1, 7).to(DEV)
+    np.random.seed(0)
+    mask = torch.from_numpy(OracleMaskGenerator(96, 96, 32, 16, 0.65)())[None]
+    vol = model.videomae._volume(x)
+    # the frozen weights' gradients as the backward writes them (before the optimiser step)
+    dp._fwd_bwd(vol, _prep_mask(mask, vol.device, None))
+    frozen_sq = sum(dp.arena.g(k).double().square().sum().item() for k in frozen)
+    dp.step(vol, _prep_mask(mask, vol.device, None))
+    trainable = []
+    for k, p in model.named_parameters():
+        if p.requires_grad:
+            trainable.append(torch.nn.Parameter(torch.empty_like(p)))
+            trainable[-1].grad = dp.arena.g(k).clone()
+    want = torch.nn.utils.clip_grad_norm_(trainable, float("inf")).item()
+    got = opt.grad_norm().item()
+    whole = (want ** 2 + frozen_sq) ** 0.5
+    print(f"clip norm with frozen parameters: {got:.6g}, clip_grad_norm_ {want:.6g}, rel {abs(got - want) / want:.2e} (bound 1e-6); "
+          f"norm including the frozen gradients {whole:.6g} (rel {abs(whole - want) / want:.2e})")
+    assert frozen_sq > 0 and abs(got - want) <= 1e-6 * want  # measured 1.2e-7 on B200 (1000 W)
+    assert abs(whole - want) >= 100 * 1e-6 * want
+
+
 def test_whole_model_reduced_precision_mode(ops, tmp_path):
     """`from_pretrained(..., torch_dtype=torch.bfloat16)` (run_inspect.py:106-111): weights held in bf16, outputs returned in
     bf16, numbers within the embedding tolerance of the fp32 oracle evaluated on the bf16-rounded weights."""
