@@ -75,6 +75,7 @@ __global__ void __launch_bounds__(256) rope3d_kernel(__nv_bfloat16* __restrict__
     }
 #pragma unroll
     for (int i = 0; i < 8; i += 2) {
+      if (e0 + i >= 3 * a.seg) continue;  // pass-through pair (3*seg is even): keep its bits, -0.0 included
       float o0, o1;
       // explicit products / fused adds: both kernels round identically (no compiler-chosen FMA contraction)
       if (!a.transpose) {
@@ -165,9 +166,10 @@ __global__ void __launch_bounds__(256, 3) rope3d_v2_kernel(__nv_bfloat16* __rest
       const int pb0 = p0 * a.half, pb1 = p1 * a.half, pb2 = p2 * a.half;
 #pragma unroll
       for (int i = 0; i < 4; ++i) {  // one adjacent pair per 32-bit word
+        const int code0 = ee[2 * i], code1 = ee[2 * i + 1];
+        if (code0 == 0xFFFF) continue;  // pass-through pair (3*seg is even, so code1 is 0xFFFF too): keep its bits, -0.0 included
         const float x0 = __uint_as_float(w[i] << 16), x1 = __uint_as_float(w[i] & 0xFFFF0000u);
         float2 a0 = make_float2(1.f, 0.f), a1 = make_float2(1.f, 0.f);
-        const int code0 = ee[2 * i], code1 = ee[2 * i + 1];
         if (fast) {
           if (code0 != 0xFFFF) a0 = cs[((code0 >> 8) == 0 ? pb0 : (code0 >> 8) == 1 ? pb1 : pb2) + (code0 & 0xFF)];
           if (code1 != 0xFFFF) a1 = cs[((code1 >> 8) == 0 ? pb0 : (code1 >> 8) == 1 ? pb1 : pb2) + (code1 & 0xFF)];

@@ -258,7 +258,10 @@ def test_vjepa_encoder_gradients_match_oracle_and_reference(small_vjepa, gold):
     # K bias: sum_j dK_j vanishes identically without the rotary map (softmax-backward rows sum to zero), so with it the
     # gradient is a small residual of cancelling bf16 dK rows: measured 5.7e-2, bound 1.5e-1; everything else 5e-2
     # (round 2, bf16 tubelet-embedding operands: worst measured 5.8e-2 on a LayerNorm weight of this deliberately ill-conditioned fixture
-    # — Q/K std 0.3 — where round 1's TF32 embedding gave 4.6e-2; bound 7e-2)
+    # — Q/K std 0.3 — where round 1's TF32 embedding gave 4.6e-2; bound 7e-2).
+    # test_gpu_vjepa_kernels.py checks the K slot stage by stage (Frobenius-rel 5.3e-3 to the true gradient given the
+    # kernels' own attention inputs) and shows why its bound cannot be derived tighter: the true K-bias gradient is only
+    # 1.6 - 4.6x the worst case of the two bf16 roundings of dK alone
     tol = lambda k: 1.5e-1 if k.endswith("key.bias") else 7e-2
     errs = sorted(((frob(got[k], osd[k].grad), k) for k in osd), reverse=True)
     assert all(e <= tol(k) for e, k in errs), errs[:4]
@@ -512,7 +515,8 @@ def test_native_predictor_gradients_match_oracle(small_vjepa_pred, gold):
         if n == "embeddings.mask_tokens":  # only the chosen token (index 1) is used
             assert float(p.grad[0].abs().max()) == 0.0
         e = frob(p.grad, ref)
-        if not e <= (1.5e-1 if n.endswith("key.bias") else 5e-2):  # K bias: a residual of cancelling bf16 dK rows (see the encoder test)
+        # K bias: a residual of cancelling bf16 dK rows (see the encoder test and test_gpu_vjepa_kernels.py)
+        if not e <= (1.5e-1 if n.endswith("key.bias") else 5e-2):
             bad[n] = e
     assert not bad, bad
     model.zero_grad(set_to_none=True)
