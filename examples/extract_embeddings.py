@@ -31,6 +31,8 @@ def main(argv=None):
     ap.add_argument("--format", default="parquet", choices=["parquet", "npy"])
     ap.add_argument("--model_id", default="smb-vision-base")
     ap.add_argument("--config_overrides", default="")
+    ap.add_argument("--layers", default="", help="comma-separated hidden-state indices (0 = patch embedding, k = block k), "
+                    "e.g. 3,6,9,12: each embedding is then [len(layers), N, d] instead of last_hidden_state")
     args = ap.parse_args(argv)
 
     from transformers import VideoMAEConfig
@@ -63,7 +65,8 @@ def main(argv=None):
     items = shard_volumes(items, rank, world)
 
     prep = VolumePreprocessor(args.image_size, args.depth, device=dev)
-    runner = EmbeddingRunner(model, preprocess=prep)
+    layers = [int(k) for k in args.layers.split(",") if k] or None
+    runner = EmbeddingRunner(model, preprocess=prep, layers=layers)
     writer = EmbeddingWriter(args.save_dir, fmt=args.format, model_id=args.model_id)
 
     def raw_stream():

@@ -63,6 +63,12 @@ int smbv_patch_embed_select_fwd(const float* volume /*[B,T,H,W]*/, const smbv_bf
  * x fp32 [M,d] (rows may be gathered through row_idx), y bf16 [M,d]; mean/rstd optional (saved for backward). */
 int smbv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, int M, int d,
                        smbv_bf16* y, float* mean /*[M] or NULL*/, float* rstd /*[M] or NULL*/, smbv_stream_t st);
+/* the same, and the fp32 input rows are also stored to x_copy [M,d] (or NULL): block k's input is the hidden state k of
+ * `output_hidden_states` (VideoMAEModel.forward returns the input of every layer and the last output), written from the registers that
+ * already hold it.  x and x_copy 16-byte aligned. */
+int smbv_layernorm_fwd_copy(const float* x, const float* gamma, const float* beta, float eps, int M, int d, smbv_bf16* y,
+                            float* mean /*[M] or NULL*/, float* rstd /*[M] or NULL*/, float* x_copy /*[M,d] or NULL*/,
+                            smbv_stream_t st);
 
 /* ---- K5, K7-K10, K12: nn.Linear (F.linear, modeling_videomae.py:262-264, :311, :368, :382, :801-803, :722) as a
  * tcgen05 GEMM  C[M,N] = A[M,K] * W[N,K]^T  (bf16 operands, fp32 accumulate in TMEM) with a fused epilogue. */
@@ -186,6 +192,12 @@ int smbv_layernorm_bwd(const smbv_bf16* dy, const float* x, const float* mean, c
                        int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16 /*or NULL*/, float* dgamma,
                        float* dbeta, float* workspace, smbv_stream_t st);
 int smbv_layernorm_bwd_blocks(void);
+/* the same with a second fp32 addend: dres = (accumulate ? dres : 0) + dLN/dx + extra, bf16 copy of that sum.  `extra` [M,d]
+ * (or NULL) is the gradient of the hidden state that enters this LayerNorm (`output_hidden_states`); no
+ * workspace. */
+int smbv_layernorm_bwd_add(const smbv_bf16* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
+                           int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16 /*or NULL*/, float* dgamma,
+                           float* dbeta, const float* extra /*[M,d] or NULL*/, smbv_stream_t st);
 
 /* ---- bias / mask-token gradients: out[n] += sum_m x[m,n]  (x row-major with leading dimension ld) */
 int smbv_colsum_bf16(const smbv_bf16* x, int M, int N, int64_t ld, float* out, smbv_stream_t st);
@@ -296,6 +308,11 @@ int smbv_l1_loss_f32(const float* pred, const float* target, int64_t n, float* w
 int smbv_cast_f32_bf16(const float* src, smbv_bf16* dst, int64_t n, smbv_stream_t st);
 /* dst[i] = scale * float(src[i])   (gradient all-reduce wire format bf16 -> fp32 master gradients, with the 1/world mean) */
 int smbv_cast_bf16_f32_scale(const smbv_bf16* src, float* dst, int64_t n, float scale, smbv_stream_t st);
+/* x[i] = (*scale_dev) * x[i] + addend[i], then x_bf16[i] = bf16(x[i]); scale_dev NULL = 1, addend NULL = 0, x_bf16 NULL =
+ * no copy.  n a multiple of 4.  The gradient of a hidden state (`output_hidden_states`) joins
+ * the residual-stream gradient at the encoder output, and the upstream d(loss) factor is applied there. */
+int smbv_scale_add_recast_f32(float* x, int64_t n, const float* scale_dev /*or NULL*/, const float* addend /*or NULL*/,
+                              smbv_bf16* x_bf16 /*or NULL*/, smbv_stream_t st);
 
 #ifdef __cplusplus
 }

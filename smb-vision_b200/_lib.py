@@ -63,6 +63,7 @@ SIGNATURES = {
     "smbv_patch_embed_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "smbv_patch_embed_select_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P],
     "smbv_layernorm_fwd": [_P, _P, _P, _F, _I, _I, _P, _P, _P, _P],
+    "smbv_layernorm_fwd_copy": [_P, _P, _P, _F, _I, _I, _P, _P, _P, _P, _P],
     "smbv_gemm_bf16": [C.POINTER(GemmArgs), _P],
     "smbv_gemm_ex": [C.POINTER(GemmExArgs), _P],
     "smbv_flash_attn_bwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P, _P, _P, _P, _P],
@@ -70,6 +71,7 @@ SIGNATURES = {
     "smbv_flash_attn_bwd_fused": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P, _P, _L, _P, _P, _P, _P, _P, _P],
     "smbv_layernorm_bwd": [_P, _P, _P, _P, _P, _I, _I, _P, _I, _P, _P, _P, _P, _P],
     "smbv_layernorm_bwd_blocks": [],
+    "smbv_layernorm_bwd_add": [_P, _P, _P, _P, _P, _I, _I, _P, _I, _P, _P, _P, _P, _P],
     "smbv_colsum_bf16": [_P, _I, _I, _L, _P, _P],
     "smbv_colsum_f32": [_P, _I, _I, _L, _P, _P],
     "smbv_colsum_heads_bf16": [_P, _I, _I, _I, _P, _I, _P],
@@ -101,6 +103,7 @@ SIGNATURES = {
     "smbv_l1_loss_f32": [_P, _P, _L, _P, _P, _P, _F, _P],
     "smbv_cast_f32_bf16": [_P, _P, _L, _P],
     "smbv_cast_bf16_f32_scale": [_P, _P, _L, _F, _P],
+    "smbv_scale_add_recast_f32": [_P, _L, _P, _P, _P, _P],
 }
 
 _lib = None
@@ -135,7 +138,7 @@ def check(rc: int, what: str) -> None:
 
 
 # kernels launched per C-ABI call (for bench.py's gpu_launches count)
-LAUNCHES_PER_CALL = {"smbv_normpix_loss": 2, "smbv_layernorm_bwd": 2, "smbv_flash_attn_bwd": 3, "smbv_flash_attn_bwd_ex": 3, "smbv_flash_attn_bwd_fused": 4, "smbv_sumsq_f32": 2, "smbv_l1_loss_f32": 2, "smbv_token_sum": 2, "smbv_attn_small_bwd": 2}
+LAUNCHES_PER_CALL = {"smbv_normpix_loss": 2, "smbv_layernorm_bwd": 2, "smbv_layernorm_bwd_add": 2, "smbv_flash_attn_bwd": 3, "smbv_flash_attn_bwd_ex": 3, "smbv_flash_attn_bwd_fused": 4, "smbv_sumsq_f32": 2, "smbv_l1_loss_f32": 2, "smbv_token_sum": 2, "smbv_attn_small_bwd": 2}
 launch_count = 0
 # optional hook(name) -> context manager, used by bench.py to bracket one kernel family with CUDA events
 event_hook = None

@@ -9,7 +9,9 @@ namespace smbv {
 // ------------------------------------------------------------------------------------------------
 // LayerNorm backward, two kernels (a fused single kernel needed ~190 registers -> 8 warps/SM):
 //  (rows)    one warp per row:  xhat = (x - mean) rstd ; g = dy * gamma ; dx = rstd (g - mean(g) - xhat mean(g xhat))
-//            dres (fp32 residual-stream gradient) (+)= dx ; optional bf16 copy of the updated dres for the next GEMM
+//            dres (fp32 residual-stream gradient) (+)= dx (+ extra) ; optional bf16 copy of the updated dres for the next GEMM.
+//            `extra` (or NULL): a second fp32 addend of the same shape — the gradient of a hidden state returned by
+//            `output_hidden_states`, which joins the residual-stream gradient at this layer boundary
 //  (columns) dgamma[c] += sum_rows dy * xhat ; dbeta[c] += sum_rows dy   (lane = 8 columns, warps stride over rows)
 // ------------------------------------------------------------------------------------------------
 template <int NV>
@@ -17,7 +19,8 @@ __global__ void __launch_bounds__(256) layernorm_bwd_rows_kernel(const __nv_bflo
                                                                  const float* __restrict__ mean, const float* __restrict__ rstd,
                                                                  const float* __restrict__ gamma, int M, int d,
                                                                  float* __restrict__ dres, int accumulate,
-                                                                 __nv_bfloat16* __restrict__ dres_bf16) {
+                                                                 __nv_bfloat16* __restrict__ dres_bf16,
+                                                                 const float* __restrict__ extra) {
   const int lane = threadIdx.x & 31;
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (row >= M) return;
@@ -27,6 +30,7 @@ __global__ void __launch_bounds__(256) layernorm_bwd_rows_kernel(const __nv_bflo
   const float4* xr = reinterpret_cast<const float4*>(x + (int64_t)row * d);
   const uint2* dyr = reinterpret_cast<const uint2*>(dy + (int64_t)row * d);
   float4* dr = reinterpret_cast<float4*>(dres + (int64_t)row * d);
+  const float4* er = extra ? reinterpret_cast<const float4*>(extra + (int64_t)row * d) : nullptr;
   float4 xh[NV], g[NV], prev[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) {  // every load of the row is issued before the first use
@@ -36,6 +40,10 @@ __global__ void __launch_bounds__(256) layernorm_bwd_rows_kernel(const __nv_bflo
     const __nv_bfloat162 d01 = *reinterpret_cast<const __nv_bfloat162*>(&dv.x), d23 = *reinterpret_cast<const __nv_bfloat162*>(&dv.y);
     g[i] = make_float4(__low2float(d01), __high2float(d01), __low2float(d23), __high2float(d23));
     prev[i] = (accumulate && c < nvec) ? dr[c] : make_float4(0.f, 0.f, 0.f, 0.f);
+    if (er && c < nvec) {
+      const float4 e = er[c];
+      prev[i] = make_float4(prev[i].x + e.x, prev[i].y + e.y, prev[i].z + e.z, prev[i].w + e.w);
+    }
   }
   float s1 = 0.f, s2 = 0.f;
 #pragma unroll
@@ -198,22 +206,16 @@ __global__ void __launch_bounds__(256) gather_patches_kernel(const float* __rest
 
 using namespace smbv;
 
-extern "C" int smbv_layernorm_bwd(const smbv_bf16* dy, const float* x, const float* mean, const float* rstd,
-                                  const float* gamma, int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16,
-                                  float* dgamma, float* dbeta, float* workspace, smbv_stream_t st) {
-  (void)workspace;  // kept in the ABI; the two-kernel version needs none
-  SMBV_ARG(dy && x && mean && rstd && gamma && dres && dgamma && dbeta, "layernorm_bwd: null pointer");
-  SMBV_ARG(M > 0 && d > 0 && d % 8 == 0 && d <= 1024, "layernorm_bwd: need d %% 8 == 0 and d <= 1024 (got M=%d d=%d)", M, d);
-  SMBV_ARG(((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dres)) & 15) == 0,
-           "layernorm_bwd: pointers must be 16-byte aligned");
+static int layernorm_bwd_launch(const smbv_bf16* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
+                                int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16, float* dgamma, float* dbeta,
+                                const float* extra, cudaStream_t s) {
   const int nv = (d / 4 + 31) / 32;
-  cudaStream_t s = (cudaStream_t)st;
   const __nv_bfloat16* dyy = reinterpret_cast<const __nv_bfloat16*>(dy);
   __nv_bfloat16* db = reinterpret_cast<__nv_bfloat16*>(dres_bf16);
   const int grid = (M + 7) / 8;
-#define LNB_CASE(NV)                                                                                           \
-  case NV:                                                                                                     \
-    layernorm_bwd_rows_kernel<NV><<<grid, 256, 0, s>>>(dyy, x, mean, rstd, gamma, M, d, dres, accumulate, db);  \
+#define LNB_CASE(NV)                                                                                                  \
+  case NV:                                                                                                            \
+    layernorm_bwd_rows_kernel<NV><<<grid, 256, 0, s>>>(dyy, x, mean, rstd, gamma, M, d, dres, accumulate, db, extra);  \
     break;
   switch (nv <= 1 ? 1 : nv <= 2 ? 2 : nv <= 3 ? 3 : nv <= 4 ? 4 : nv <= 6 ? 6 : 8) {
     LNB_CASE(1) LNB_CASE(2) LNB_CASE(3) LNB_CASE(4) LNB_CASE(6) LNB_CASE(8)
@@ -224,6 +226,30 @@ extern "C" int smbv_layernorm_bwd(const smbv_bf16* dy, const float* x, const flo
   layernorm_bwd_params_kernel<<<pgrid, 256, 0, s>>>(dyy, x, mean, rstd, M, d, dgamma, dbeta);
   SMBV_LAUNCH_CHECK("layernorm_bwd_params");
   return 0;
+}
+
+extern "C" int smbv_layernorm_bwd(const smbv_bf16* dy, const float* x, const float* mean, const float* rstd,
+                                  const float* gamma, int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16,
+                                  float* dgamma, float* dbeta, float* workspace, smbv_stream_t st) {
+  (void)workspace;  // kept in the ABI; the two-kernel version needs none
+  SMBV_ARG(dy && x && mean && rstd && gamma && dres && dgamma && dbeta, "layernorm_bwd: null pointer");
+  SMBV_ARG(M > 0 && d > 0 && d % 8 == 0 && d <= 1024, "layernorm_bwd: need d %% 8 == 0 and d <= 1024 (got M=%d d=%d)", M, d);
+  SMBV_ARG(((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dres)) & 15) == 0,
+           "layernorm_bwd: pointers must be 16-byte aligned");
+  return layernorm_bwd_launch(dy, x, mean, rstd, gamma, M, d, dres, accumulate, dres_bf16, dgamma, dbeta, nullptr,
+                              (cudaStream_t)st);
+}
+
+extern "C" int smbv_layernorm_bwd_add(const smbv_bf16* dy, const float* x, const float* mean, const float* rstd,
+                                      const float* gamma, int M, int d, float* dres, int accumulate, smbv_bf16* dres_bf16,
+                                      float* dgamma, float* dbeta, const float* extra, smbv_stream_t st) {
+  SMBV_ARG(dy && x && mean && rstd && gamma && dres && dgamma && dbeta, "layernorm_bwd_add: null pointer");
+  SMBV_ARG(M > 0 && d > 0 && d % 8 == 0 && d <= 1024, "layernorm_bwd_add: need d %% 8 == 0 and d <= 1024 (got M=%d d=%d)", M, d);
+  SMBV_ARG(((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dres) |
+             reinterpret_cast<uintptr_t>(extra)) & 15) == 0,
+           "layernorm_bwd_add: pointers must be 16-byte aligned");
+  return layernorm_bwd_launch(dy, x, mean, rstd, gamma, M, d, dres, accumulate, dres_bf16, dgamma, dbeta, extra,
+                              (cudaStream_t)st);
 }
 
 extern "C" int smbv_layernorm_bwd_blocks(void) { return 4 * num_sms(); }

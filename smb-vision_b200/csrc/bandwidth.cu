@@ -88,12 +88,14 @@ __global__ void sincos_kernel(float* __restrict__ out, int n, int d) {
 
 // ------------------------------------------------------------------------------------------------
 // LayerNorm forward: one warp per row, the row lives in registers (NV float4 per lane), two-pass statistics.
+// x_copy (or NULL): the input row is also stored there — the per-layer hidden state of `output_hidden_states`, taken from
+// the registers of block k's first LayerNorm instead of a second pass over the residual stream.
 // ------------------------------------------------------------------------------------------------
 template <int NV>
 __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, float eps, int M, int d,
                                                             __nv_bfloat16* __restrict__ y, float* __restrict__ mean_out,
-                                                            float* __restrict__ rstd_out) {
+                                                            float* __restrict__ rstd_out, float* __restrict__ x_copy) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= M) return;
   const int lane = threadIdx.x & 31;
@@ -106,6 +108,12 @@ __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const float* __restr
     int c = lane + 32 * i;
     v[i] = c < nvec ? xr[c] : make_float4(0.f, 0.f, 0.f, 0.f);
     s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
+  }
+  if (x_copy) {
+    float4* xc = reinterpret_cast<float4*>(x_copy + (int64_t)row * d);
+#pragma unroll
+    for (int i = 0; i < NV; ++i)
+      if (lane + 32 * i < nvec) xc[lane + 32 * i] = v[i];
   }
   const float mean = warp_sum(s) / (float)d;
   float q = 0.f;
@@ -390,6 +398,24 @@ __global__ void cast_bf16_f32_scale_kernel(const __nv_bfloat16* __restrict__ src
   }
 }
 
+// x = scale * x + addend, then the bf16 copy of the result (every part optional).  Joins the gradient of a returned hidden
+// state to the residual-stream gradient at a boundary that has no LayerNorm backward pass, and applies the upstream
+// d(loss) factor there (device scalar: no host synchronisation).
+__global__ void scale_add_recast_kernel(float* __restrict__ x, int64_t n4, const float* __restrict__ scale,
+                                        const float* __restrict__ addend, __nv_bfloat16* __restrict__ x_bf16) {
+  const float sc = scale ? *scale : 1.f;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    float4 v = reinterpret_cast<const float4*>(x)[i];
+    if (scale) v = make_float4(sc * v.x, sc * v.y, sc * v.z, sc * v.w);
+    if (addend) {
+      const float4 a = reinterpret_cast<const float4*>(addend)[i];
+      v = make_float4(v.x + a.x, v.y + a.y, v.z + a.z, v.w + a.w);
+    }
+    reinterpret_cast<float4*>(x)[i] = v;
+    if (x_bf16) reinterpret_cast<uint2*>(x_bf16)[i] = make_uint2(pack_bf16(v.x, v.y), pack_bf16(v.z, v.w));
+  }
+}
+
 }  // namespace smbv
 
 using namespace smbv;
@@ -423,17 +449,14 @@ extern "C" int smbv_sincos_table(float* out, int n, int d, smbv_stream_t st) {
   return 0;
 }
 
-extern "C" int smbv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, int M, int d,
-                                  smbv_bf16* y, float* mean, float* rstd, smbv_stream_t st) {
-  SMBV_ARG(x && gamma && beta && y, "layernorm_fwd: null pointer");
-  SMBV_ARG(M > 0 && d > 0 && d % 4 == 0 && d <= 4096, "layernorm_fwd: need d %% 4 == 0 and d <= 4096 (got M=%d d=%d)", M, d);
+static int layernorm_fwd_launch(const float* x, const float* gamma, const float* beta, float eps, int M, int d, smbv_bf16* y,
+                                float* mean, float* rstd, float* x_copy, cudaStream_t s) {
   const int nv = (d / 4 + 31) / 32;
   dim3 grid((M + 7) / 8), block(256);
-  cudaStream_t s = (cudaStream_t)st;
   __nv_bfloat16* yy = reinterpret_cast<__nv_bfloat16*>(y);
-#define LN_CASE(NV)                                                                                    \
-  case NV:                                                                                             \
-    layernorm_fwd_kernel<NV><<<grid, block, 0, s>>>(x, gamma, beta, eps, M, d, yy, mean, rstd);        \
+#define LN_CASE(NV)                                                                                         \
+  case NV:                                                                                                  \
+    layernorm_fwd_kernel<NV><<<grid, block, 0, s>>>(x, gamma, beta, eps, M, d, yy, mean, rstd, x_copy);     \
     break;
   switch (nv <= 1 ? 1 : nv <= 2 ? 2 : nv <= 3 ? 3 : nv <= 4 ? 4 : nv <= 6 ? 6 : nv <= 8 ? 8 : nv <= 16 ? 16 : 32) {
     LN_CASE(1) LN_CASE(2) LN_CASE(3) LN_CASE(4) LN_CASE(6) LN_CASE(8) LN_CASE(16) LN_CASE(32)
@@ -441,6 +464,22 @@ extern "C" int smbv_layernorm_fwd(const float* x, const float* gamma, const floa
 #undef LN_CASE
   SMBV_LAUNCH_CHECK("layernorm_fwd");
   return 0;
+}
+
+extern "C" int smbv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, int M, int d,
+                                  smbv_bf16* y, float* mean, float* rstd, smbv_stream_t st) {
+  SMBV_ARG(x && gamma && beta && y, "layernorm_fwd: null pointer");
+  SMBV_ARG(M > 0 && d > 0 && d % 4 == 0 && d <= 4096, "layernorm_fwd: need d %% 4 == 0 and d <= 4096 (got M=%d d=%d)", M, d);
+  return layernorm_fwd_launch(x, gamma, beta, eps, M, d, y, mean, rstd, nullptr, (cudaStream_t)st);
+}
+
+extern "C" int smbv_layernorm_fwd_copy(const float* x, const float* gamma, const float* beta, float eps, int M, int d,
+                                       smbv_bf16* y, float* mean, float* rstd, float* x_copy, smbv_stream_t st) {
+  SMBV_ARG(x && gamma && beta && y, "layernorm_fwd_copy: null pointer");
+  SMBV_ARG(M > 0 && d > 0 && d % 4 == 0 && d <= 4096, "layernorm_fwd_copy: need d %% 4 == 0 and d <= 4096 (got M=%d d=%d)", M, d);
+  SMBV_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(x_copy)) & 15) == 0,
+           "layernorm_fwd_copy: x and x_copy must be 16-byte aligned");
+  return layernorm_fwd_launch(x, gamma, beta, eps, M, d, y, mean, rstd, x_copy, (cudaStream_t)st);
 }
 
 extern "C" int smbv_fill_mask_tokens(float* x_dec, const float* mask_token, const float* pos, const int32_t* msk_idx,
@@ -517,5 +556,19 @@ extern "C" int smbv_cast_bf16_f32_scale(const smbv_bf16* src, float* dst, int64_
   cast_bf16_f32_scale_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, (cudaStream_t)st>>>(
       reinterpret_cast<const __nv_bfloat16*>(src), dst, n, scale);
   SMBV_LAUNCH_CHECK("cast_bf16_f32_scale");
+  return 0;
+}
+
+extern "C" int smbv_scale_add_recast_f32(float* x, int64_t n, const float* scale_dev, const float* addend, smbv_bf16* x_bf16,
+                                         smbv_stream_t st) {
+  SMBV_ARG(x, "scale_add_recast_f32: null pointer");
+  SMBV_ARG(n > 0 && n % 4 == 0, "scale_add_recast_f32: n=%lld must be a positive multiple of 4", (long long)n);
+  SMBV_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(addend)) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(x_bf16) & 7) == 0,
+           "scale_add_recast_f32: x and addend must be 16-byte aligned, x_bf16 8-byte aligned");
+  const int64_t n4 = n / 4, want = (n4 + 255) / 256, cap = (int64_t)num_sms() * 8;
+  scale_add_recast_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, (cudaStream_t)st>>>(
+      x, n4, scale_dev, addend, reinterpret_cast<__nv_bfloat16*>(x_bf16));
+  SMBV_LAUNCH_CHECK("scale_add_recast_f32");
   return 0;
 }

@@ -177,11 +177,12 @@ def _pack_layer(layer: _Layer, heads: int, eps: float, arena=None, prefix: str =
     return p
 
 
-def _block_forward(X: torch.Tensor, p: _PackedLayer, rope=None) -> None:
+def _block_forward(X: torch.Tensor, p: _PackedLayer, rope=None, x_copy=None) -> None:
     """One pre-LN transformer block, in place on the fp32 residual stream X [B, n, d]  (reference :405-431).
-    `rope` = (grid_size, ids or None, max_pos): V-JEPA's rotary embedding of Q and K (modeling_vjepa.py:346-348)."""
+    `rope` = (grid_size, ids or None, max_pos): V-JEPA's rotary embedding of Q and K (modeling_vjepa.py:346-348).
+    `x_copy`: fp32 like X, receives the block's input (stored by the first LayerNorm, which reads X anyway)."""
     B, n, d = X.shape
-    h = ops.layernorm_fwd(X, p.g1, p.be1, p.eps)
+    h = ops.layernorm_fwd(X, p.g1, p.be1, p.eps, x_copy=x_copy)
     pad32 = p.hd == 32 and getattr(p, "pad32", False)
     if rope is not None and p.hd != 64 and not pad32:
         raise SmbvError("the rotary embedding kernel is wired to the tcgen05 attention paths (head_dim 64, or 32 zero-padded)")
@@ -242,6 +243,24 @@ def _prep_mask(bool_masked_pos: torch.Tensor, device, num_masked: Optional[int])
         if not bool((c[:, 1] == num_masked).all()):
             raise RuntimeError("bool_masked_pos must mask the same number of patches for every sample in the batch")
     return fine, vis, msk, slot, N - num_masked, num_masked
+
+
+def _check_layers(layers, L: int):
+    """hidden-state indices 0..L (0 = patch embedding, L = last block)."""
+    layers = [int(k) for k in layers]
+    bad = [k for k in layers if not 0 <= k <= L]
+    if bad:
+        raise ValueError(f"hidden-state indices {bad} outside 0..{L} (0 = patch embedding, {L} = last block)")
+    return layers
+
+
+def _want_states(output_hidden_states, config) -> bool:
+    """`output_hidden_states=None` falls back to `config.output_hidden_states` (upstream PreTrainedModel semantics)."""
+    return bool(_cfg(config, "output_hidden_states", False) if output_hidden_states is None else output_hidden_states)
+
+
+def _out_states(states, dtype):
+    return tuple(states) if dtype is None else tuple(h.to(dtype) for h in states)
 
 
 class _PretrainedIO:
@@ -470,9 +489,12 @@ class B200VideoMAEModel(_PretrainedIO, nn.Module):
         v = pixel_values.to(device=dev, dtype=torch.float32, non_blocking=True)
         return v.reshape(B, T, H, W).contiguous()  # C == 1: permute(0,2,1,3,4) of reference :190 is free
 
-    def encode(self, vol: torch.Tensor, mask_pack=None, blend: bool = False) -> torch.Tensor:
+    def encode(self, vol: torch.Tensor, mask_pack=None, blend: bool = False, keep=None):
         """fp32 volume [B,T,H,W] -> fp32 residual stream [B, n, d] after all encoder blocks.  `blend`: SimMIM style — masked
-        tokens are replaced by the encoder mask token in the patch-embed epilogue and all N tokens are kept."""
+        tokens are replaced by the encoder mask token in the patch-embed epilogue and all N tokens are kept.
+        `keep`: hidden-state indices (0 = patch embedding, k = output of block k-1, taken before the final LayerNorm) ->
+        returns (X, states) with states[k] fp32 [B, n, d] for k in `keep` and None elsewhere (num_hidden_layers + 1 entries);
+        state L is the residual stream itself, the others are copies written by the first LayerNorm of the next block."""
         self._check_config()
         pk = self.packed()
         pos = self.pos_table(self.config.hidden_size, vol.device)
@@ -485,11 +507,18 @@ class B200VideoMAEModel(_PretrainedIO, nn.Module):
         else:
             fine, _, _, slot, n_vis, _ = mask_pack
             X = ops.patch_embed_fwd(vol, pk["wpe16"], pk["bpe"], pos, fine, slot, n_vis)
-        for p in pk["layers"]:
-            _block_forward(X, p)
+        L = len(pk["layers"])
+        keep = None if keep is None else set(_check_layers(keep, L))
+        states = [None] * (L + 1)
+        for i, p in enumerate(pk["layers"]):
+            if keep is not None and i in keep:
+                states[i] = torch.empty_like(X)
+            _block_forward(X, p, x_copy=states[i])
+        if keep is not None and L in keep:
+            states[L] = X
         if self.layernorm is not None:  # use_mean_pooling=False only (reference :517-520, :648-649)
             X = ops.layernorm_fwd(X, _f32(self.layernorm.weight), _f32(self.layernorm.bias), self.config.layer_norm_eps).float()
-        return X
+        return X if keep is None else (X, states)
 
     def forward(self, pixel_values, bool_masked_pos=None, head_mask=None, output_attentions=None,
                 output_hidden_states=None, return_dict=None, num_masked: Optional[int] = None, **kwargs):
@@ -500,18 +529,32 @@ class B200VideoMAEModel(_PretrainedIO, nn.Module):
         with torch.no_grad():
             vol = self._volume(pixel_values)
             mp = None if bool_masked_pos is None else _prep_mask(bool_masked_pos, vol.device, num_masked)
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            from .training import encoder_autograd_forward  # one autograd node: CUDA forward with saves + hand-scheduled backward
-
-            X = encoder_autograd_forward(self, vol, mp)
-        else:
-            with torch.no_grad():
-                X = self.encode(vol, mp)
+        X, states = self._encode_states(vol, mp, _want_states(output_hidden_states, self.config))
         if self._out_dtype is not None:
             X = X.to(self._out_dtype)
+        hs = None
+        if states is not None:  # upstream: the last state IS last_hidden_state when no final LayerNorm follows
+            hs = _out_states(states[:-1], self._out_dtype) + ((X,) if self.layernorm is None else _out_states(states[-1:], self._out_dtype))
         if return_dict is False:
-            return (X,)
-        return BaseModelOutput(last_hidden_state=X, hidden_states=None, attentions=None)
+            return (X,) if hs is None else (X, hs)
+        return BaseModelOutput(last_hidden_state=X, hidden_states=hs, attentions=None)
+
+    def _encode_states(self, vol, mask_pack, want: bool):
+        """-> (X, states or None): the encoder output (after the final LayerNorm, if any) and, with `want`, the
+        num_hidden_layers + 1 hidden states (the last one before that LayerNorm).  Differentiable when grad is enabled and a
+        parameter requires it (one autograd node: CUDA forward with saves + hand-scheduled backward)."""
+        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            from .training import encoder_autograd_forward
+
+            out = encoder_autograd_forward(self, vol, mask_pack, states=want)
+            if not want:
+                return out, None
+            X, states = out[0], list(out[1:])
+            return X, (states + [X] if self.layernorm is None else states)
+        with torch.no_grad():
+            if not want:
+                return self.encode(vol, mask_pack), None
+            return self.encode(vol, mask_pack, keep=range(self.config.num_hidden_layers + 1))
 
 
 class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
@@ -580,9 +623,11 @@ class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
             # reference :868-874 raises for C != 3 when norm_pix_loss is False
             raise ValueError("Can't unnormalize non-RGB images. Consider setting config.norm_pix_loss to False.")
 
-    def forward_no_grad(self, vol: torch.Tensor, mask_pack, want_dlogits: bool = False):
-        """Forward of reference :791-897 on device tensors.  Returns (loss, logits bf16 [B,n_mask,K], dlogits|None)."""
+    def forward_no_grad(self, vol: torch.Tensor, mask_pack, want_dlogits: bool = False, states: bool = False):
+        """Forward of reference :791-897 on device tensors.  Returns (loss, logits bf16 [B,n_mask,K], dlogits|None), and the
+        encoder's hidden states as a fourth item with `states`."""
         self._check_config()
+        keep = range(self.config.num_hidden_layers + 1) if states else None
         c = self.config
         fine, vis, msk, slot, n_vis, n_mask = mask_pack
         B = vol.shape[0]
@@ -590,7 +635,8 @@ class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
         pk = self.packed()
         pos_d = self.videomae.pos_table(dd, vol.device)
         if self.mim_style == "simmim":
-            X = self.videomae.encode(vol, mask_pack, blend=True)  # [B, N, d] fp32, masked rows = mask token + PE
+            X = self.videomae.encode(vol, mask_pack, blend=True, keep=keep)  # [B, N, d] fp32, masked rows = mask token + PE
+            X, hs = X if states else (X, None)
             Xb = ops.cast_bf16(X)
             Xd = torch.empty((B, N, dd), dtype=torch.float32, device=vol.device)
             every = torch.arange(N, dtype=torch.int32, device=vol.device)
@@ -602,8 +648,9 @@ class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
             hN = ops.layernorm_fwd(G, pk["gn"], pk["bn"], 1e-5)
             logits = ops.gemm(hN, pk["wh"], pk["bh"], ops.EPI_BF16)
             loss, dlogits = ops.normpix_loss(vol, msk, n_mask, logits, want_dlogits, self.loss_kind, c.patch_size)
-            return loss, logits, dlogits
-        X = self.videomae.encode(vol, mask_pack)  # [B, n_vis, d] fp32
+            return (loss, logits, dlogits, hs) if states else (loss, logits, dlogits)
+        X = self.videomae.encode(vol, mask_pack, keep=keep)  # [B, n_vis, d] fp32
+        X, hs = X if states else (X, None)
         Xb = ops.cast_bf16(X)
         Xd = torch.empty((B, N, dd), dtype=torch.float32, device=vol.device)
         for b in range(B):  # visible rows: encoder_to_decoder + PE[vis]  (reference :801-811, :815)
@@ -616,7 +663,7 @@ class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
             ops.layernorm_fwd(Xd[b, n_vis:], pk["gn"], pk["bn"], 1e-5, out=hN[b])
         logits = ops.gemm(hN, pk["wh"], pk["bh"], ops.EPI_BF16)  # [B, n_mask, 4096] bf16 (reference :722)
         loss, dlogits = ops.normpix_loss(vol, msk, n_mask, logits, want_dlogits, self.loss_kind, c.patch_size)
-        return loss, logits, dlogits
+        return (loss, logits, dlogits, hs) if states else (loss, logits, dlogits)
 
     def forward(self, pixel_values, bool_masked_pos=None, head_mask=None, output_attentions=None,
                 output_hidden_states=None, return_dict=None, num_masked: Optional[int] = None, **kwargs):
@@ -629,17 +676,22 @@ class B200VideoMAEForPreTraining(_PretrainedIO, nn.Module):
         with torch.no_grad():
             vol = self.videomae._volume(pixel_values)
             mp = _prep_mask(bool_masked_pos, vol.device, num_masked)
+        want = _want_states(output_hidden_states, self.config)
+        hs = None
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             from .training import autograd_forward  # differentiable path: one autograd node around the CUDA fwd/bwd
 
             self.refresh_operands()
-            loss, logits = autograd_forward(self, vol, mp)
+            loss, logits, *states = autograd_forward(self, vol, mp, states=want)
         else:
             with torch.no_grad():
-                loss, logits, _ = self.forward_no_grad(vol, mp)
+                loss, logits, _, *states = self.forward_no_grad(vol, mp, states=want)
+                states = states[0] if want else []
+        if want:  # the encoder's states (visible tokens; all N for mim_style="simmim")
+            hs = _out_states(states, self._out_dtype)
         if return_dict is False:
-            return (loss, logits)
-        return VideoMAEForPreTrainingOutput(loss=loss, logits=logits, hidden_states=None, attentions=None)
+            return (loss, logits) if hs is None else (loss, logits, hs)
+        return VideoMAEForPreTrainingOutput(loss=loss, logits=logits, hidden_states=hs, attentions=None)
 
 
 class B200VideoMAEForVideoClassification(_PretrainedIO, nn.Module):
@@ -714,14 +766,20 @@ class B200VideoMAEForVideoClassification(_PretrainedIO, nn.Module):
         with torch.no_grad():
             vol = self.videomae._volume(pixel_values)
             feats, lab = self._prep(additional_features, labels, vol.device)
+        want = _want_states(output_hidden_states, self.config)
+        states = None
         if lab is not None and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             from .training import cls_autograd_forward
 
             self.videomae.refresh_operands()
-            loss, logits = cls_autograd_forward(self, vol, feats, lab)
+            loss, logits, *states = cls_autograd_forward(self, vol, feats, lab, states=want)
         else:
+            if want:  # without labels there is no loss to train, but the states stay differentiable under grad
+                X, states = self.videomae._encode_states(vol, None, True)
             with torch.no_grad():
-                X = self.videomae.encode(vol, None)  # [B, N, d] fp32 (already through videomae.layernorm if not mean pooling)
+                if not want:
+                    X = self.videomae.encode(vol, None)  # [B, N, d] fp32 (already through videomae.layernorm if not mean pooling)
+                X = X.detach()
                 hp = self.head_params()
                 if self.fc_norm is not None:  # reference :974-975
                     pooled, inv_n = ops.token_sum(X), 1.0 / X.shape[1]
@@ -731,6 +789,7 @@ class B200VideoMAEForVideoClassification(_PretrainedIO, nn.Module):
                                                self.problem_id(lab))
         if self._out_dtype is not None:
             logits = logits.to(self._out_dtype)
+        hs = _out_states(states, self._out_dtype) if want else None
         if return_dict is False:
-            return ((loss, logits) if loss is not None else (logits,))
-        return ImageClassifierOutput(loss=loss, logits=logits, hidden_states=None, attentions=None)
+            return tuple(v for v in (loss, logits, hs) if v is not None)
+        return ImageClassifierOutput(loss=loss, logits=logits, hidden_states=hs, attentions=None)

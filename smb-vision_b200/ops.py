@@ -113,8 +113,9 @@ def patch_embed_select_fwd(volume, weight, bias, pos, fine, mask_token) -> torch
     return out
 
 
-def layernorm_fwd(x, gamma, beta, eps: float, save_stats: bool = False, out=None):
-    """x fp32 [..., d] -> bf16 [..., d] (+ mean, rstd fp32 [M] when save_stats)."""
+def layernorm_fwd(x, gamma, beta, eps: float, save_stats: bool = False, out=None, x_copy=None):
+    """x fp32 [..., d] -> bf16 [..., d] (+ mean, rstd fp32 [M] when save_stats).  x_copy: fp32 like x, receives a copy of x
+    (written from the registers the LayerNorm reads x into)."""
     _chk(x, torch.float32, "x")
     _chk(gamma, torch.float32, "gamma")
     _chk(beta, torch.float32, "beta")
@@ -125,7 +126,13 @@ def layernorm_fwd(x, gamma, beta, eps: float, save_stats: bool = False, out=None
     if save_stats:
         mean = torch.empty((M,), dtype=torch.float32, device=x.device)
         rstd = torch.empty((M,), dtype=torch.float32, device=x.device)
-    call("smbv_layernorm_fwd", _ptr(x), _ptr(gamma), _ptr(beta), float(eps), M, d, _ptr(y), _ptr(mean), _ptr(rstd), _stream())
+    if x_copy is None:
+        call("smbv_layernorm_fwd", _ptr(x), _ptr(gamma), _ptr(beta), float(eps), M, d, _ptr(y), _ptr(mean), _ptr(rstd), _stream())
+    else:
+        if _chk(x_copy, torch.float32, "x_copy").shape != x.shape:
+            raise SmbvError(f"layernorm_fwd: x_copy must be shaped like x {tuple(x.shape)}")
+        call("smbv_layernorm_fwd_copy", _ptr(x), _ptr(gamma), _ptr(beta), float(eps), M, d, _ptr(y), _ptr(mean), _ptr(rstd),
+             _ptr(x_copy), _stream())
     return (y, mean, rstd) if save_stats else y
 
 
@@ -282,17 +289,23 @@ def qkv_wgrad(dqkv, x, dw, tokens, heads, batch_index=0, batch=1):
 _ln_ws = {}
 
 
-def layernorm_bwd(dy, x, mean, rstd, gamma, dres, accumulate, dgamma, dbeta, want_bf16=True):
-    """dres (+)= dLN/dx; returns the bf16 copy of the updated dres (or None)."""
+def layernorm_bwd(dy, x, mean, rstd, gamma, dres, accumulate, dgamma, dbeta, want_bf16=True, extra=None):
+    """dres (+)= dLN/dx (+ extra, fp32 like x); returns the bf16 copy of the updated dres (or None)."""
     _chk(dy, torch.bfloat16, "dy")
     _chk(x, torch.float32, "x")
     _chk(dres, torch.float32, "dres")
     d = x.shape[-1]
     M = x.numel() // d
+    db = torch.empty(x.shape, dtype=torch.bfloat16, device=x.device) if want_bf16 else None
+    if extra is not None:
+        if _chk(extra, torch.float32, "extra").shape != x.shape:
+            raise SmbvError(f"layernorm_bwd: extra must be shaped like x {tuple(x.shape)}")
+        call("smbv_layernorm_bwd_add", _ptr(dy), _ptr(x), _ptr(mean), _ptr(rstd), _ptr(gamma), M, d, _ptr(dres),
+             1 if accumulate else 0, _ptr(db), _ptr(dgamma), _ptr(dbeta), _ptr(extra), _stream())
+        return db
     key = (str(x.device), d)
     if key not in _ln_ws:
         _ln_ws[key] = torch.empty((_lib.load().smbv_layernorm_bwd_blocks() * 2 * d,), dtype=torch.float32, device=x.device)
-    db = torch.empty(x.shape, dtype=torch.bfloat16, device=x.device) if want_bf16 else None
     call("smbv_layernorm_bwd", _ptr(dy), _ptr(x), _ptr(mean), _ptr(rstd), _ptr(gamma), M, d, _ptr(dres), 1 if accumulate else 0,
          _ptr(db), _ptr(dgamma), _ptr(dbeta), _ptr(_ln_ws[key]), _stream())
     return db
@@ -329,6 +342,19 @@ def cast_f32_scaled(src: torch.Tensor, dst: torch.Tensor, scale: float) -> torch
     _chk(dst, torch.float32, "dst")
     call("smbv_cast_bf16_f32_scale", _ptr(src), _ptr(dst), src.numel(), float(scale), _stream())
     return dst
+
+
+def scale_add_recast_(x: torch.Tensor, scale: Optional[torch.Tensor] = None, addend: Optional[torch.Tensor] = None,
+                      want_bf16: bool = True):
+    """x = scale * x + addend in place (scale: a 1-element tensor, moved to the device as fp32 without a host sync; None = 1;
+    addend fp32 like x or None); returns the bf16 copy of the result (or None)."""
+    _chk(x, torch.float32, "x")
+    if addend is not None and _chk(addend, torch.float32, "addend").shape != x.shape:
+        raise SmbvError(f"scale_add_recast_: addend must be shaped like x {tuple(x.shape)}")
+    sc = None if scale is None else scale.detach().to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+    xb = torch.empty(x.shape, dtype=torch.bfloat16, device=x.device) if want_bf16 else None
+    call("smbv_scale_add_recast_f32", _ptr(x), x.numel(), _ptr(sc), _ptr(addend), _ptr(xb), _stream())
+    return xb
 
 
 # measurement hook (bench.py): a callable returning two raw cudaEvent_t handles that the library records around the dK/dV

@@ -383,13 +383,15 @@ def block_forward_train(X, p, rope=None) -> Tuple[torch.Tensor, _BlockSaved]:
 
 
 def block_backward(dX, dXb, s: _BlockSaved, p, arena, prefix: str, names: Optional[Dict[str, object]] = None, rope=None,
-                   sq: Optional[SideQueue] = None):
+                   sq: Optional[SideQueue] = None, extra=None):
     """dX: fp32 [B,n,d] gradient of the block output (updated IN PLACE to the gradient of the block input);
     dXb: its bf16 copy.  Returns the bf16 copy of the updated dX.  `names`: role -> parameter name (default: the VideoMAE
     block under `prefix`); `rope`: as in block_forward_train — the gradients of the rotated Q, K go back through the
     transposed rotary map before the bias / weight / input gradients are formed.  `sq`: the caller's SideQueue — weight / bias
     gradients are queued there (each AFTER the critical-path kernel that starts from the same inputs has been launched); the
-    caller closes the block with `sq.block_done` and ends with `sq.finish()`.  None = everything on the current stream."""
+    caller closes the block with `sq.block_done` and ends with `sq.finish()`.  None = everything on the current stream.
+    `extra`: fp32 like dX or None — the gradient of the block's input as a returned hidden state, added by the last LayerNorm
+    backward (so both the updated dX and its bf16 copy include it)."""
     B, n, d = dX.shape
     H = p.heads
     g = arena.g
@@ -458,7 +460,7 @@ def block_backward(dX, dXb, s: _BlockSaved, p, arena, prefix: str, names: Option
         for b in range(B):
             ops.qkv_dgrad(dqkv, p.wqkv, n, H, batch_index=b, batch=B, out=dh1[b])
         qkv_wb(mk, dqkv, H)
-    dXb = ops.layernorm_bwd(dh1, s.x_in, s.m1, s.r1, p.g1, dX, True, g(nm["ln1w"]), g(nm["ln1b"]))
+    dXb = ops.layernorm_bwd(dh1, s.x_in, s.m1, s.r1, p.g1, dX, True, g(nm["ln1w"]), g(nm["ln1b"]), extra=extra)
     return dXb
 
 
@@ -501,16 +503,19 @@ def encoder_forward_train(vm, vol, mask_pack=None, blend: bool = False):
 
 
 def encoder_backward(vm, vol, saved, dX, dXb, arena: GradArena, idx, n_sel: int, done: Callable[[], None], blend_pack=None,
-                     sq: Optional[SideQueue] = None):
+                     sq: Optional[SideQueue] = None, dhidden=None):
     """dX fp32 [B,n,d] (+ bf16 copy) = gradient of the encoder output -> encoder-block and patch-embedding gradients.
     `idx` int32 [B, >= n_sel]: the tokens that reached the encoder (the visible ones; all of them without a mask).
-    `sq`: the caller's SideQueue (its `done` closes the blocks on it and the caller finishes it)."""
+    `sq`: the caller's SideQueue (its `done` closes the blocks on it and the caller finishes it).
+    `dhidden`: gradients of the hidden states (fp32 [B,n,d] or None, index k = input of block k); entry k joins dX in
+    block k's last LayerNorm backward.  Entries past the last block are the caller's (already in dX)."""
     pe = vm.packed()
     g = arena.g
     d = vm.config.hidden_size
     patches, blocks = saved[0], saved[1:]
     for i in reversed(range(len(blocks))):
-        dXb = block_backward(dX, dXb, blocks[i], pe["layers"][i], arena, f"videomae.encoder.layer.{i}.", sq=sq)
+        dXb = block_backward(dX, dXb, blocks[i], pe["layers"][i], arena, f"videomae.encoder.layer.{i}.", sq=sq,
+                             extra=None if dhidden is None else dhidden[i])
         done()
     if blend_pack is not None:
         # SimMIM blend: E[b,n] = mask ? mask_token : conv(P[n]) + bias — the masked rows of dE sum into the mask token, the
@@ -527,8 +532,15 @@ def encoder_backward(vm, vol, saved, dX, dXb, arena: GradArena, idx, n_sel: int,
     done()
 
 
-def mim_forward_train(model, vol, mask_pack):
-    """Forward of reference :791-897 keeping activations.  Returns (loss, logits, dlogits, saved)."""
+def _encoder_states(S, X):
+    """The encoder's hidden states (upstream `output_hidden_states`): every block's input — kept out of place by
+    block_forward_train anyway — and the last block's output X, before the optional final LayerNorm."""
+    return [sv.x_in for sv in S.enc[1:]] + [X]
+
+
+def mim_forward_train(model, vol, mask_pack, states: bool = False):
+    """Forward of reference :791-897 keeping activations.  Returns (loss, logits, dlogits, saved); with `states`, saved.states
+    holds the encoder's hidden states."""
     model._check_config()
     vm = model.videomae
     vm._check_config()
@@ -540,6 +552,8 @@ def mim_forward_train(model, vol, mask_pack):
     pd = model.packed()
     simmim = getattr(model, "mim_style", "mae") == "simmim"
     X, S.enc = encoder_forward_train(vm, vol, mask_pack, blend=simmim)
+    if states:
+        S.states = _encoder_states(S, X)
     if vm.layernorm is not None:  # use_mean_pooling=False: final encoder LayerNorm (reference :517-520, :648-649)
         _final_ln_forward(vm, X, S)
     else:
@@ -573,9 +587,13 @@ def mim_forward_train(model, vol, mask_pack):
     return loss, logits, dlogits, S
 
 
-def mim_backward(model, S, dlogits, arena: GradArena, on_bucket: Optional[Callable[[int], None]] = None):
+def mim_backward(model, S, dlogits, arena: GradArena, on_bucket: Optional[Callable[[int], None]] = None, dhidden=None,
+                 loss_scale=None):
     """Backward of the whole model into `arena` (gradients are ACCUMULATED: zero the arena first for a fresh step).
-    `on_bucket(i)` is called as soon as bucket i of `order_groups` is complete (DP all-reduce hook)."""
+    `on_bucket(i)` is called as soon as bucket i of `order_groups` is complete (DP all-reduce hook).
+    `dhidden` (list of num_hidden_layers + 1 fp32 tensors or None): gradients of the encoder's hidden states, added at their
+    layer boundaries; the gradients are then loss_scale * d(loss) + the hidden-state terms — the loss gradient is scaled
+    where it enters the encoder, and the decoder / head gradients behind it at the end."""
     vm = model.videomae
     c = model.config
     fine, vis, msk, slot, n_vis, n_mask = S.mask_pack
@@ -628,41 +646,70 @@ def mim_backward(model, S, dlogits, arena: GradArena, on_bucket: Optional[Callab
     ge2d = g("encoder_to_decoder.weight")
     sq.run(mk, lambda: ops.linear_wgrad(dZb, S.xb, ge2d), dZb, S.xb)
     done()
-    dXb = ops.cast_bf16(dX)
+    if dhidden is None:
+        dXb = ops.cast_bf16(dX)
+    else:  # loss gradient * loss_scale (+ the last hidden state's gradient when no final LayerNorm follows it)
+        dXb = ops.scale_add_recast_(dX, loss_scale, dhidden[-1] if vm.layernorm is None else None)
     if vm.layernorm is not None:  # back through the final encoder LayerNorm
-        dX, dXb = _final_ln_backward(vm, S, dXb, arena)
-    encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, vis, n_vis, done, blend_pack=S.mask_pack if simmim else None, sq=sq)
+        dX, dXb = _final_ln_backward(vm, S, dXb, arena, extra=None if dhidden is None else dhidden[-1])
+    encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, vis, n_vis, done, blend_pack=S.mask_pack if simmim else None, sq=sq,
+                     dhidden=dhidden)
     sq.finish()
+    if dhidden is not None:  # the loss-only gradients (head, decoder, mask_token, encoder_to_decoder: the buckets before the encoder's)
+        ops.scale_f32_(arena.flat[:arena.bucket_bounds[c.decoder_num_hidden_layers + 2]], loss_scale)
 
 
 # ----------------------------------------------------------------------------------------------
 # autograd bridge (HF Trainer / plain loss.backward())
 # ----------------------------------------------------------------------------------------------
+def _hidden_grads(ctx, dH):
+    """The gradients of the returned hidden states as contiguous fp32 tensors (None where unused), or None when all are
+    unused.  Reading ctx.saved_tensors raises torch's in-place modification error if a returned state was edited: the
+    hand-written backward reads the same tensors."""
+    ctx.saved_tensors
+    if all(g is None for g in dH):
+        return None
+    return [None if g is None else g.float().contiguous() for g in dH]
+
+
+def _loss_scale(grad_loss, device):
+    return torch.zeros(1, dtype=torch.float32, device=device) if grad_loss is None else grad_loss
+
+
 class _MIMFunction(torch.autograd.Function):
     """One node for the whole model: forward runs the CUDA forward, backward runs `mim_backward` and hands every
-    parameter its gradient, so `out.loss.backward()` works exactly like with the reference module."""
+    parameter its gradient, so `out.loss.backward()` works exactly like with the reference module.  With `states` the
+    encoder's hidden states are further outputs, differentiable through the same backward."""
 
     @staticmethod
-    def forward(ctx, model, vol, mask_pack, names, *params):
-        loss, logits, dlogits, S = mim_forward_train(model, vol, mask_pack)
+    def forward(ctx, model, vol, mask_pack, names, states, *params):
+        loss, logits, dlogits, S = mim_forward_train(model, vol, mask_pack, states=states)
         ctx.model, ctx.S, ctx.dlogits, ctx.names = model, S, dlogits, names
         ctx.needs = [p.requires_grad for p in params]
         ctx.mark_non_differentiable(logits)
-        return loss, logits
+        ctx.set_materialize_grads(False)
+        hs = S.states if states else []
+        ctx.save_for_backward(*hs)
+        return (loss, logits, *hs)
 
     @staticmethod
-    def backward(ctx, grad_loss, _grad_logits):
+    def backward(ctx, grad_loss, _grad_logits, *dH):
         arena = GradArena(ctx.model, ctx.S.vol.device)  # fresh: autograd may adopt these views as p.grad
-        mim_backward(ctx.model, ctx.S, ctx.dlogits, arena)  # gradients for d(loss) = 1; the saved dlogits stay untouched
-        # upstream factor (gradient accumulation, loss scaling; 1.0 for a plain .backward()) applied in fp32 on the way out
-        ops.scale_f32_(arena.flat, grad_loss)
+        dhidden = _hidden_grads(ctx, dH)
+        if dhidden is None:
+            mim_backward(ctx.model, ctx.S, ctx.dlogits, arena)  # gradients for d(loss) = 1; the saved dlogits stay untouched
+            # upstream factor (gradient accumulation, loss scaling; 1.0 for a plain .backward()) applied in fp32 on the way out
+            ops.scale_f32_(arena.flat, grad_loss)
+        else:  # the factor must not reach the hidden-state terms: mim_backward applies it to the loss gradient only
+            mim_backward(ctx.model, ctx.S, ctx.dlogits, arena, dhidden=dhidden, loss_scale=_loss_scale(grad_loss, arena.flat.device))
         grads = tuple(arena.views[n] if need else None for n, need in zip(ctx.names, ctx.needs))
-        return (None, None, None, None) + grads
+        return (None, None, None, None, None) + grads
 
 
-def autograd_forward(model, vol, mask_pack):
+def autograd_forward(model, vol, mask_pack, states: bool = False):
+    """-> (loss, logits[, hidden state 0, ..., hidden state L])."""
     names, params = zip(*model.named_parameters())
-    return _MIMFunction.apply(model, vol, mask_pack, list(names), *params)
+    return _MIMFunction.apply(model, vol, mask_pack, list(names), states, *params)
 
 
 class _EncoderOnly(torch.nn.Module):
@@ -681,36 +728,50 @@ def _final_ln_forward(vm, X, S):
     return S.xb
 
 
-def _final_ln_backward(vm, S, dYb, arena):
-    """dYb bf16 [B,n,d] = gradient of the final LayerNorm's output -> (dX fp32, dX bf16) of its input."""
+def _final_ln_backward(vm, S, dYb, arena, extra=None):
+    """dYb bf16 [B,n,d] = gradient of the final LayerNorm's output -> (dX fp32, dX bf16) of its input (+ `extra`, the
+    gradient of that input as the last hidden state)."""
     dX = torch.empty_like(S.x_pre)
     dXb = ops.layernorm_bwd(dYb, S.x_pre, S.mE, S.rE, vm.layernorm.weight.detach(), dX, False,
-                            arena.g("videomae.layernorm.weight"), arena.g("videomae.layernorm.bias"))
+                            arena.g("videomae.layernorm.weight"), arena.g("videomae.layernorm.bias"), extra=extra)
     return dX, dXb
 
 
 class _EncoderFunction(torch.autograd.Function):
     """`model.videomae(x[, mask]).last_hidden_state` with gradients (reference VideoMAEModel.forward, :537-658, under
-    autograd): forward = the CUDA forward keeping activations, backward = `encoder_backward`."""
+    autograd): forward = the CUDA forward keeping activations, backward = `encoder_backward`.  With `states` the hidden
+    states are further outputs: every block's input, and the last block's output when a final LayerNorm follows it (without
+    one that output is X itself)."""
 
     @staticmethod
-    def forward(ctx, vm, vol, mask_pack, names, *params):
+    def forward(ctx, vm, vol, mask_pack, names, states, *params):
         S = _ModelSaved()
         X, S.enc = encoder_forward_train(vm, vol, mask_pack)
+        hs = _encoder_states(S, X) if states else []
         if vm.layernorm is not None:
             X = _final_ln_forward(vm, X, S).float()
+        elif hs:
+            hs.pop()  # state L is the returned X
         S.vol, S.mask_pack = vol, mask_pack
-        ctx.vm, ctx.S, ctx.names = vm, S, names
+        ctx.vm, ctx.S, ctx.names, ctx.x_shape = vm, S, names, X.shape
         ctx.needs = [p.requires_grad for p in params]
-        return X
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(*hs)
+        return (X, *hs) if states else X
 
     @staticmethod
-    def backward(ctx, dOut):
+    def backward(ctx, dOut, *dH):
         vm, S = ctx.vm, ctx.S
         arena = GradArena(_EncoderOnly(vm), S.vol.device)
-        B, n = dOut.shape[:2]
+        dhidden = _hidden_grads(ctx, dH)
+        if dhidden is not None and vm.layernorm is None:
+            dhidden.append(None)  # the last state is X: its gradient is dOut
+        B, n = ctx.x_shape[:2]
+        if dOut is None:  # only hidden states were used
+            dOut = torch.zeros(ctx.x_shape, dtype=torch.float32, device=S.vol.device)
         if vm.layernorm is not None:
-            dX, dXb = _final_ln_backward(vm, S, ops.cast_bf16(dOut.float().contiguous()), arena)
+            dX, dXb = _final_ln_backward(vm, S, ops.cast_bf16(dOut.float().contiguous()), arena,
+                                         extra=None if dhidden is None else dhidden[-1])
         else:
             dX = dOut.float().clone()  # the block backward updates it in place
             dXb = ops.cast_bf16(dX)
@@ -718,15 +779,16 @@ class _EncoderFunction(torch.autograd.Function):
             idx = torch.arange(n, dtype=torch.int32, device=dX.device).repeat(B, 1).contiguous()
         else:
             idx = S.mask_pack[1]
-        encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, idx, n, lambda: None)
+        encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, idx, n, lambda: None, dhidden=dhidden)
         grads = tuple(arena.views["videomae." + nm] if need else None for nm, need in zip(ctx.names, ctx.needs))
-        return (None, None, None, None) + grads
+        return (None, None, None, None, None) + grads
 
 
-def encoder_autograd_forward(vm, vol, mask_pack):
+def encoder_autograd_forward(vm, vol, mask_pack, states: bool = False):
+    """-> X, or (X, hidden states ...) with `states` (see _EncoderFunction)."""
     vm.refresh_operands()
     names, params = zip(*vm.named_parameters())
-    return _EncoderFunction.apply(vm, vol, mask_pack, list(names), *params)
+    return _EncoderFunction.apply(vm, vol, mask_pack, list(names), states, *params)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -875,13 +937,16 @@ class DataParallelStep:
 # ----------------------------------------------------------------------------------------------
 # classification fine-tuning (SURVEY.md §8f rank 1; reference VideoMAEForVideoClassification :917-1023)
 # ----------------------------------------------------------------------------------------------
-def cls_forward_train(model, vol, feats, labels, arena: GradArena):
+def cls_forward_train(model, vol, feats, labels, arena: GradArena, states: bool = False):
     """Encoder (all tokens, no mask) -> token mean -> fc_norm -> [cat features] -> classifier -> loss.  The head's own
     gradients (classifier, fc_norm) are produced by the same launch as its forward and land in `arena`.
-    Returns (loss, logits fp32 [B,L], dpooled fp32 [B,d], saved)."""
+    Returns (loss, logits fp32 [B,L], dpooled fp32 [B,d], saved); with `states`, saved.states holds the encoder's hidden
+    states."""
     vm = model.videomae
     S = _ModelSaved()
     X, S.enc = encoder_forward_train(vm, vol, None)
+    if states:
+        S.states = _encoder_states(S, X)
     B, N, d = X.shape
     hp = model.head_params()
     grads = dict(dW=arena.g("classifier.weight"), dbias=arena.g("classifier.bias"),
@@ -896,8 +961,9 @@ def cls_forward_train(model, vol, feats, labels, arena: GradArena):
     return loss, logits, dpooled, S
 
 
-def cls_backward(model, S, dpooled, arena: GradArena, on_bucket: Optional[Callable[[int], None]] = None):
-    """Broadcast d(loss)/d(mean token) to every token row, then the encoder / patch-embedding backward."""
+def cls_backward(model, S, dpooled, arena: GradArena, on_bucket: Optional[Callable[[int], None]] = None, dhidden=None):
+    """Broadcast d(loss)/d(mean token) to every token row, then the encoder / patch-embedding backward.  `dhidden`: as in
+    mim_backward (the caller scales dpooled and the head's gradients)."""
     bucket = 0
     sq = SideQueue(S.vol.device)
 
@@ -912,34 +978,47 @@ def cls_backward(model, S, dpooled, arena: GradArena, on_bucket: Optional[Callab
     vm = model.videomae
     if model.fc_norm is not None:
         dX, dXb = ops.broadcast_rows(dpooled, S.n)  # d mean / d token, every row
+        if dhidden is not None and dhidden[-1] is not None:
+            dXb = ops.scale_add_recast_(dX, None, dhidden[-1])
     else:  # only the first token's row of the final LayerNorm output carries gradient
         dYb = torch.zeros((B, S.n, dpooled.shape[1]), dtype=torch.bfloat16, device=dpooled.device)
         dYb[:, 0] = ops.cast_bf16(dpooled)
-        dX, dXb = _final_ln_backward(vm, S, dYb, arena)
+        dX, dXb = _final_ln_backward(vm, S, dYb, arena, extra=None if dhidden is None else dhidden[-1])
     idx = torch.arange(S.n, dtype=torch.int32, device=S.vol.device).repeat(B, 1).contiguous()
-    encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, idx, S.n, done, sq=sq)
+    encoder_backward(vm, S.vol, S.enc, dX, dXb, arena, idx, S.n, done, sq=sq, dhidden=dhidden)
     sq.finish()
 
 
 class _ClsFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, model, vol, feats, labels, names, *params):
+    def forward(ctx, model, vol, feats, labels, names, states, *params):
         arena = GradArena(model, vol.device)
-        loss, logits, dpooled, S = cls_forward_train(model, vol, feats, labels, arena)
+        loss, logits, dpooled, S = cls_forward_train(model, vol, feats, labels, arena, states=states)
         ctx.model, ctx.S, ctx.dpooled, ctx.names, ctx.arena = model, S, dpooled, names, arena
         ctx.needs = [p.requires_grad for p in params]
         ctx.mark_non_differentiable(logits)
-        return loss, logits
+        ctx.set_materialize_grads(False)
+        hs = S.states if states else []
+        ctx.save_for_backward(*hs)
+        return (loss, logits, *hs)
 
     @staticmethod
-    def backward(ctx, grad_loss, _grad_logits):
+    def backward(ctx, grad_loss, _grad_logits, *dH):
         arena = ctx.arena
-        cls_backward(ctx.model, ctx.S, ctx.dpooled, arena)  # everything for d(loss) = 1 (head gradients came with the forward)
-        ops.scale_f32_(arena.flat, grad_loss)
+        dhidden = _hidden_grads(ctx, dH)
+        if dhidden is None:
+            cls_backward(ctx.model, ctx.S, ctx.dpooled, arena)  # everything for d(loss) = 1 (head gradients came with the forward)
+            ops.scale_f32_(arena.flat, grad_loss)
+        else:  # the upstream factor scales the loss seed and the head's gradients, not the hidden-state terms
+            sc = _loss_scale(grad_loss, arena.flat.device)
+            dpooled = ops.scale_f32_(ctx.dpooled.clone(), sc)
+            cls_backward(ctx.model, ctx.S, dpooled, arena, dhidden=dhidden)
+            ops.scale_f32_(arena.flat[:arena.bucket_bounds[1]], sc)  # bucket 0: classifier (+ fc_norm)
         grads = tuple(arena.views[n] if need else None for n, need in zip(ctx.names, ctx.needs))
-        return (None, None, None, None, None) + grads
+        return (None, None, None, None, None, None) + grads
 
 
-def cls_autograd_forward(model, vol, feats, labels):
+def cls_autograd_forward(model, vol, feats, labels, states: bool = False):
+    """-> (loss, logits[, hidden state 0, ..., hidden state L])."""
     names, params = zip(*model.named_parameters())
-    return _ClsFunction.apply(model, vol, feats, labels, list(names), *params)
+    return _ClsFunction.apply(model, vol, feats, labels, list(names), states, *params)
